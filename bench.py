@@ -1,7 +1,7 @@
 #!/usr/bin/env python3
 """Benchmark of the geometry-decoding hot path (latents -> occupancy grid -> mesh).
 
-    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config hier|dense] [--res R]
+    python bench.py --gpus N --steps K --warmup W [--impl reference] [--config hier|dense] [--res R] [--dump-outputs DIR]
     torchrun --nnodes=1 --nproc-per-node N ... bench.py --gpus N --steps K --warmup W
 
 Default workload = BASELINE.json configs[2], the configuration the metric ("latents->mesh ms and query pts/sec @octree
@@ -26,9 +26,20 @@ Metric: decoder query points per second over the whole job = (queries the algori
               refinement (4 n_c^3 + 4 n_f^3 + 8 A bytes per level) and of marching cubes (4 N^3 + 12 V + 12 F).
 ``cpu_baseline`` / ``--impl reference``: the oracle port of the reference PyTorch fp32 path on the host cores, bounded
               sample (the reference tree itself is absent on the GPU box).
+
+``--dump-outputs DIR`` writes what the last timed step computed (rank 0) as DIR/<name>.npy, every value finite:
+``latents`` (ShapeVAE.forward, [tokens, width]); ``grid_visited`` (the volume decoder's grid at the points it evaluated, rows
+of (flat grid index, logit): the sparse decoders leave NaN at the others; skipped while the grid stays sharded over the
+ranks); ``mesh_v`` / ``mesh_f`` (the marching-cubes mesh without the non-finite vertices along the rim of the visited band
+and the faces using them, as ``export_to_trimesh`` / ``MCSurfaceExtractor(cull_nonfinite=True)`` return it).  The inputs
+are seeded, so two builds run with the same arguments can be compared output for output.  See ``dump_outputs`` for the
+size cap.
+
+bench.py writes nothing into the source tree (which may be read-only): no byte-code caches, no build products.
 """
 import argparse
 import json
+import math
 import os
 import subprocess
 import sys
@@ -40,6 +51,7 @@ import torch
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True       # the project's modules are imported from the tree: leave no __pycache__ there
 
 METRIC = "decoder_query_points_per_sec"
 UNIT = "pts/s"
@@ -130,6 +142,33 @@ def cpu_port_rate(cfg, sd, lat, seconds, min_chunks=2, res=96):
     return n / dt, done, torch.get_num_threads()
 
 
+DUMP_BYTES = 63 * 10 ** 6             # array data; the .npy headers stay well inside the last MB of the 64 MB cap
+
+
+def dump_outputs(out_dir, arrays, limit=DUMP_BYTES):
+    """Writes each tensor of ``arrays`` (name -> tensor, None skipped) as ``out_dir/<name>.npy``: float64 as float64, other
+    floating point as float32, integers as float64 (exact for int32).  The tensors are written smallest first and each may
+    take an equal share of what is left of ``limit``; one that does not fit is cut to a sample of its rows (dim 0) drawn
+    with a fixed seed, so the same shape always keeps the same rows, in their original order."""
+    os.makedirs(out_dir, exist_ok=True)
+    todo = []
+    for name, t in arrays.items():
+        if t is not None:
+            dt = torch.float32 if t.is_floating_point() and t.dtype != torch.float64 else torch.float64
+            todo.append((t.numel() * dt.itemsize, name, t, dt))
+    todo.sort(key=lambda x: x[0])
+    left = limit
+    for i, (_, name, t, dt) in enumerate(todo):
+        row_bytes = math.prod(t.shape[1:]) * dt.itemsize
+        keep = min(t.shape[0], left // (len(todo) - i) // row_bytes)
+        if keep < t.shape[0]:
+            rows = np.sort(np.random.default_rng(0).choice(t.shape[0], keep, replace=False))
+            t = t[torch.from_numpy(rows).to(t.device)]
+        a = t.to(dt).cpu().numpy()
+        np.save(os.path.join(out_dir, name + ".npy"), a)
+        left -= a.nbytes
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
@@ -145,7 +184,13 @@ def main():
                     help="multiply the decoder's q_norm / k_norm gains (1.3-1.4 puts the weight-only score bound above 15.9: shows the "
                          "attention kernel's floor with per-head shifts on; changes the field, so a tuning run, not the headline)")
     ap.add_argument("--gather", action="store_true", help="N > 1: gather the grid instead of keeping it sharded through marching cubes")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write what the last timed step computed as DIR/<name>.npy (float32 / float64, at most 64 MB in all)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs writes the outputs of the device path (--impl ours)")
     res = args.res if args.res is not None else (384 if args.config == "hier" else 256)
 
     rank = int(os.environ.get("RANK", "0"))
@@ -234,14 +279,19 @@ def main():
     mesh_size = [0, 0]
 
     tf_group = True if world > 1 else None        # N > 1: the latent transformer runs sequence-parallel over the ranks
+    last = {}                                     # --dump-outputs: what the latest step_device computed
 
     def step_device():
         lat = vae(z_dev, group=tf_group)
         grid = vae.volume_decoder(lat, vae.geo_decoder, **kw)
+        m = None
         if grid is not None:
             m = vae.surface_extractor.run_device(grid[0], mc_level=0.0, bounds=1.01, octree_resolution=res)
             if m is not None:
                 mesh_size[0], mesh_size[1] = m[0].shape[0], m[1].shape[0]
+        if args.dump_outputs:
+            last.update(latents=lat.reshape(-1, lat.shape[-1]), grid=grid[0].reshape(-1) if isinstance(grid, torch.Tensor) else None,
+                        mesh=m)
 
     def step_e2e():
         outs = vae.latents2mesh(vae(z_host.to(dev, non_blocking=True), group=tf_group), **kw)
@@ -280,6 +330,14 @@ def main():
         sampler.start()
     ms, launches, _ = timed(step_device, args.steps)
     clocks = sampler.summary() if sampler else None
+    if args.dump_outputs and rank == 0:
+        out = {"latents": last["latents"]}
+        if last["grid"] is not None:
+            visited = torch.nonzero(torch.isfinite(last["grid"])).flatten()
+            out["grid_visited"] = torch.stack([visited.double(), last["grid"][visited].double()], 1)
+        if last["mesh"] is not None:
+            out["mesh_v"], out["mesh_f"] = ctx.mesh_clean(*last["mesh"], flip_winding=False)
+        dump_outputs(args.dump_outputs, out)
     # per-family device times from a separate profiled pass (CUDA events around every launch perturb the step by ~1 %)
     ms_prof, _, prof = timed(step_device, min(args.steps, 5), profile=True)
     prof_steps = min(args.steps, 5)

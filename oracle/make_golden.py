@@ -98,8 +98,9 @@ def main():
         report.append(f"decoder[{tag}] oracle-vs-reference max|d| logits {d_dec:.2e}  transformer {d_lat:.2e} "
                       f"(|lat|max {float(lat.abs().max()):.1f})")
         assert d_dec < 2e-5 and d_lat < 2e-3 * max(1.0, float(lat.abs().max()) / 50)
+        step = max(8, lat.shape[1] // 192)                        # at most 192 token rows: every file stays under 1 MB
         np.savez_compressed(os.path.join(GOLD, f"decoder_{tag}.npz"),
-                            queries=q.numpy(), logits=ref.numpy(), latents_out_rows=lat[0, ::8].numpy(),
+                            queries=q.numpy(), logits=ref.numpy(), latents_out_rows=lat[0, ::step].numpy(),
                             weight_checksum=checksum(sd), seed=0, latent_seed=1234)
 
     # ------------------------------------------- FlashVDM processors (selection)

@@ -1,10 +1,11 @@
 import os, sys, numpy as np, torch
-sys.path.insert(0, '/root/repo')
+ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
+sys.path.insert(0, ROOT)
 import hy3dgeo
 from hy3dgeo import weights as W, _lib
 from hy3dgeo.volume_decoders import FlashVDMVolumeDecoding
 dev = torch.device('cuda:0')
-g = np.load('/root/repo/tests/golden/volume_decoder_mini.npz')
+g = np.load(os.path.join(ROOT, 'tests', 'golden', 'volume_decoder_mini.npz'))
 cfg = W.MINI
 gain = float(g["gain"])
 sd = W.sparsify_field(W.synthetic_state_dict(cfg, seed=0), cfg, int(g["keep_freqs"]), gain, float(g["bias"]))
