@@ -103,6 +103,9 @@ SYMBOLS = {
                                      C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_float)]),
     "hy3d_mc_emit_slab": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_double), C.POINTER(C.c_double),
                                     C.c_int32, C.c_int64, c_f32p, c_i32p]),
+    "hy3d_dmc_count": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32,
+                                 C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_float)]),
+    "hy3d_dmc_emit": (C.c_int, [C.c_void_p, c_f32p, c_i32p]),
     "hy3d_mesh_clean": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int32, c_f32p, c_i32p,
                                   C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "hy3d_profile": (C.c_int, [C.c_void_p, C.c_int]),
@@ -550,6 +553,19 @@ class GeoContext:
         m = (C.c_double * 3)(*[float(v) for v in mul])
         a = (C.c_double * 3)(*[float(v) for v in add])
         self._check(self.lib.hy3d_mc_emit_slab(self.h, d, m, a, int(plane0), int(id_base), _ptr(verts), _ptr(faces)), "hy3d_mc_emit_slab")
+
+    def dmc_count(self, grid: torch.Tensor):
+        """Dual marching cubes, phase 1 (see hy3dgeo.h): -> (nV, nF, (min, max, nan)) of the fp32 grid, inside iff > 0."""
+        self.sync_stream()
+        nv, nf = C.c_int64(), C.c_int64()
+        mm = (C.c_float * 3)()
+        self._check(self.lib.hy3d_dmc_count(self.h, _ptr(grid), grid.shape[0], grid.shape[1], grid.shape[2],
+                                            C.byref(nv), C.byref(nf), mm), "hy3d_dmc_count")
+        return nv.value, nf.value, (mm[0], mm[1], bool(mm[2]))
+
+    def dmc_emit(self, verts: torch.Tensor, faces: torch.Tensor):
+        self.sync_stream()
+        self._check(self.lib.hy3d_dmc_emit(self.h, _ptr(verts), _ptr(faces)), "hy3d_dmc_emit")
 
     def mesh_clean(self, verts: torch.Tensor, faces: torch.Tensor, flip_winding: bool):
         """Device tensors (verts float32 [V,3], faces int32 [F,3]) -> the same mesh without non-finite / unreferenced

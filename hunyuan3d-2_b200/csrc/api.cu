@@ -148,6 +148,7 @@ void hy3d_destroy(hy3d_ctx* ctx) {
   ctx->kv.k32.release(); ctx->kv.v32.release(); ctx->kv.ktile.release(); ctx->kv.vtile.release();
   ctx->kv.head_shift.release(); ctx->kv.redo.release();
   ctx->mc.bits.release(); ctx->mc.rowcnt.release(); ctx->mc.rowoff.release(); ctx->mc.stats.release();
+  { DmcState& d = ctx->dmc; for (DevBuf* b : {&d.bits, &d.rowcnt, &d.rowoff, &d.stats, &d.rec}) b->release(); }
   for (auto& b : ctx->ws) b.release();
   { TransformerState& t = ctx->tf; for (DevBuf* b : {&t.tc, &t.f32, &t.x, &t.ta, &t.tq, &t.to, &t.th, &t.kt, &t.vt, &t.st, &t.tz}) b->release(); }
   ctx->w.fold.release();

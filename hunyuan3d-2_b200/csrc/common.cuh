@@ -104,6 +104,14 @@ struct McState {
   DevBuf bits, rowcnt, rowoff, stats;
 };
 
+struct DmcState {                     // dual marching cubes (dmc.cu): hy3d_dmc_count -> hy3d_dmc_emit
+  bool counted = false;
+  const float* grid = nullptr;
+  int n0 = 0, n1 = 0, n2 = 0, words = 0;
+  long long nV = 0, nF = 0;
+  DevBuf bits, rowcnt, rowoff, stats, rec;
+};
+
 // Per-kernel-family device timing with CUDA events on the launch stream (bench.py roofline).
 enum { FAM_EMBED = 0, FAM_GEMM_QPROJ, FAM_LN, FAM_GEMM_CQ, FAM_ATTN, FAM_GEMM_CPROJ, FAM_GEMM_FC, FAM_GEMM_MLP, FAM_HEAD,
        FAM_MC_BITS, FAM_MC_ROWCOUNT, FAM_MC_SCAN, FAM_MC_EMIT, FAM_OCTREE, FAM_KV, FAM_SELECT, FAM_COUNT };
@@ -128,6 +136,7 @@ struct hy3d_ctx {
   KVSelState kvsel;
   TransformerState tf;
   McState mc;
+  DmcState dmc;
   DevBuf ws[12];                      // decoder workspaces
   DevBuf scratch, scratch2;           // octree / misc
   DevBuf ln_mr;                       // per-row (mean, rstd) of the LayerNorm folded into the running GEMM

@@ -149,27 +149,36 @@ class MCSurfaceExtractor(SurfaceExtractor):
 
 
 class DMCSurfaceExtractor(SurfaceExtractor):
-    """Second entry of the ``mc_algo`` registry (reference :79-94): dual marching cubes through the third-party ``diso``
-    package (``diso.DiffDMC``, not vendored by the reference, absent from this image).  hy3dgeo does not re-implement it
-    (SURVEY §8f rank 4, DESIGN.md §7): where ``diso`` is importable this class drives it exactly as the reference does —
-    ``sdf = -logits / octree_resolution``, ``normalize=True``, vertices re-centred on their bounding box, winding reversed —
-    and where it is not, ``run`` raises the reference's ImportError, so the item becomes ``None`` as it does there.
-    NaN voxels (sparse decoders) are passed through untouched, as in the reference."""
+    """Second entry of the ``mc_algo`` registry (reference :79-94, which calls the third-party ``diso.DiffDMC`` on
+    ``sdf = -logits / octree_resolution`` with ``normalize=True``, re-centres the vertices on their bounding box and
+    reverses the winding) as device kernels: classify -> count -> emit, dual marching cubes at iso-value 0 of that sdf,
+    i.e. inside iff ``logit > 0``.  One vertex per iso-surface patch of every cube (the mean of its edge crossings, the
+    grid spanning the unit cube), one quad — two triangles — per sign-change edge whose four cubes lie inside the grid,
+    oriented like ``MCSurfaceExtractor``'s mesh so that ``export_to_trimesh``'s flip serves both; vertices centred on
+    their bounding box.  ``mc_level`` and ``bounds`` play no part, as in the reference.  NaN voxels count as outside;
+    vertices on their rim come out NaN, as with ``mc``.  The contract is ``oracle/dmc.py``; diso's own triangles, vertex
+    order and quad split are not reproduced (DESIGN.md §2).  A ``SlabGrid`` is gathered to one tensor first."""
 
-    def run(self, grid_logit, *, octree_resolution, **kwargs):
+    def run_device(self, grid_logit, **kwargs):
+        """Returns device tensors (verts float32 [V,3], faces int32 [F,3])."""
         if type(grid_logit).__name__ == "SlabGrid":
             grid_logit = grid_logit.to_tensor()[0]
-        if not hasattr(self, "dmc"):
-            try:
-                from diso import DiffDMC
-            except ImportError:
-                raise ImportError("Please install diso via `pip install diso`, or set mc_algo to 'mc'")
-            self.dmc = DiffDMC(dtype=torch.float32).to(grid_logit.device)
-        sdf = (-grid_logit / octree_resolution).to(torch.float32).contiguous()
-        verts, faces = self.dmc(sdf, deform=None, return_quads=False, normalize=True)
-        lo, hi = verts.min(dim=0)[0], verts.max(dim=0)[0]
-        verts = verts - 0.5 * (lo + hi)                       # center_vertices (:29-34)
-        return verts.detach().cpu().numpy(), faces.detach().cpu().numpy()[:, ::-1]
+        if not isinstance(grid_logit, torch.Tensor) or not grid_logit.is_cuda:
+            raise RuntimeError("DMCSurfaceExtractor needs a CUDA tensor (hy3dgeo has no CPU path)")
+        if grid_logit.dim() != 3:
+            raise ValueError("Input volume should be a 3D array.")
+        grid = grid_logit.detach().to(torch.float32).contiguous()
+        ctx = get_context(grid.device)
+        nv, nf, _ = ctx.dmc_count(grid)
+        if nv == 0:
+            raise RuntimeError("No surface found: the grid has no sign change.")
+        verts = torch.empty((nv, 3), dtype=torch.float32, device=grid.device)
+        faces = torch.empty((nf, 3), dtype=torch.int32, device=grid.device)
+        ctx.dmc_emit(verts, faces)
+        return verts, faces
+
+    def run(self, grid_logit, **kwargs):
+        return _to_host(*self.run_device(grid_logit, **kwargs))
 
 
 def export_to_trimesh(mesh_output, device=None):

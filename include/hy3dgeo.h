@@ -232,6 +232,20 @@ int hy3d_mc_count_slab(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n
                        int64_t* h_num_verts, int64_t* h_num_faces, float h_minmax[3]);
 int hy3d_mc_emit_slab(hy3d_ctx* ctx, const double h_div[3], const double h_mul[3], const double h_add[3], int32_t plane0,
                       int64_t id_base, float* d_verts, int32_t* d_faces);
+/* ---- dual marching cubes: replaces DMCSurfaceExtractor.run (surface_extractors.py:79-94), i.e. diso.DiffDMC(sdf =
+ * -logits / res, normalize=True) + center_vertices (:29-34) + the reversed winding ------------------------------------
+ * Phase 1: classify + count.  d_grid: fp32 [n0,n1,n2]; inside test `g > 0` (iso-value 0 of sdf = -logit / res), NaN =>
+ * outside.  Returns in HOST variables the vertex count (one per iso-surface patch of every cube, the patches of
+ * mc_tables.inc's loops), the face count (two per sign-change edge whose four cubes lie inside the grid) and the finite
+ * min/max of the field, h_minmax[2] = 1 if the grid holds NaN (synchronises the stream once). */
+int hy3d_dmc_count(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n1, int32_t n2, int64_t* h_num_verts,
+                   int64_t* h_num_faces, float h_minmax[3]);
+/* Phase 2: emit the mesh of the grid given to the last hy3d_dmc_count.  Vertex = mean of its patch's edge crossings
+ * (float64, divided by n_axis - 1 per axis: the grid spans the unit cube), rounded to fp32, then centred on the bounding
+ * box of the non-NaN vertices in fp32; vertices in lexicographic (cube, patch) order, faces (two triangles per quad) in
+ * lexicographic (edge owner voxel, edge axis) order, oriented like hy3d_mc_emit's.  d_verts: fp32 [V,3]; d_faces:
+ * int32 [F,3]. */
+int hy3d_dmc_emit(hy3d_ctx* ctx, float* d_verts, int32_t* d_faces);
 /* ---- mesh clean-up: the device side of export_to_trimesh (hy3dgen/shapegen/pipelines.py:95-110) ---------------------
  * `mesh_f[:, ::-1]` (flip_winding != 0) and what trimesh.Trimesh(v, f)'s default processing does to a mesh with
  * non-finite vertices: faces that reference a NaN / inf vertex are dropped, then vertices that are non-finite or no longer
