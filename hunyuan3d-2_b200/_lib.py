@@ -108,6 +108,10 @@ SYMBOLS = {
     "hy3d_dmc_emit": (C.c_int, [C.c_void_p, c_f32p, c_i32p]),
     "hy3d_mesh_clean": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int32, c_f32p, c_i32p,
                                   C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "hy3d_mesh_remove_floaters": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int64, c_f32p, c_i32p,
+                                            C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "hy3d_mesh_weld": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, c_f32p, c_i32p,
+                                 C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "hy3d_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "hy3d_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "hy3d_debug_watchdog": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
@@ -577,6 +581,28 @@ class GeoContext:
         self._check(self.lib.hy3d_mesh_clean(self.h, _ptr(verts), verts.shape[0], _ptr(faces), faces.shape[0], int(bool(flip_winding)),
                                              _ptr(vo), _ptr(fo), C.byref(nv), C.byref(nf)), "hy3d_mesh_clean")
         return vo[: nv.value], fo[: nf.value]
+
+    def _mesh_filter(self, name, verts, faces, *args):
+        self.sync_stream()
+        verts = verts.detach().to(device=self.device, dtype=torch.float32).contiguous()
+        faces = faces.detach().to(device=self.device, dtype=torch.int32).contiguous()
+        if verts.dim() != 2 or verts.shape[1] != 3 or faces.dim() != 2 or faces.shape[1] != 3:
+            raise ValueError(f"{name}: expected verts [V, 3] and faces [F, 3], got {tuple(verts.shape)} and {tuple(faces.shape)}")
+        vo, fo = torch.empty_like(verts), torch.empty_like(faces)
+        nv, nf = C.c_int64(), C.c_int64()
+        self._check(getattr(self.lib, name)(self.h, _ptr(verts), verts.shape[0], _ptr(faces), faces.shape[0], *args,
+                                            _ptr(vo), _ptr(fo), C.byref(nv), C.byref(nf)), name)
+        return vo[: nv.value], fo[: nf.value]
+
+    def mesh_remove_floaters(self, verts: torch.Tensor, faces: torch.Tensor, min_faces: int):
+        """Device tensors -> the mesh without the faces of edge-connected components of fewer than ``min_faces`` faces and
+        without the faces touching their vertices; unreferenced vertices dropped, order kept (hy3dgeo.h)."""
+        return self._mesh_filter("hy3d_mesh_remove_floaters", verts, faces, int(min_faces))
+
+    def mesh_weld(self, verts: torch.Tensor, faces: torch.Tensor):
+        """Device tensors -> the mesh with bit-equal finite vertices merged into the smallest id, faces that collapse
+        removed, unreferenced vertices dropped, order kept (hy3dgeo.h)."""
+        return self._mesh_filter("hy3d_mesh_weld", verts, faces)
 
     def mc_cases(self, grid: torch.Tensor, level: float) -> torch.Tensor:
         self.sync_stream()

@@ -254,6 +254,24 @@ int hy3d_dmc_emit(hy3d_ctx* ctx, float* d_verts, int32_t* d_faces);
  * variables (synchronises the stream once). */
 int hy3d_mesh_clean(hy3d_ctx* ctx, const float* d_verts, int64_t nV, const int32_t* d_faces, int64_t nF, int32_t flip_winding,
                     float* d_verts_out, int32_t* d_faces_out, int64_t* h_num_verts_out, int64_t* h_num_faces_out);
+/* ---- mesh post-processing: FloaterRemover / DegenerateFaceRemover (hy3dgen/shapegen/postprocessors.py) --------------------
+ * Same buffers, output order and single synchronisation as hy3d_mesh_clean (no winding flip): surviving faces keep their
+ * order and winding, vertices are kept iff a surviving face references them, in their original order.  Vertex and face ids
+ * above int32 return HY3D_ERR_UNSUPPORTED; a face index outside [0, nV) is never dereferenced and returns HY3D_ERR_ARG; a
+ * mesh that becomes empty returns counts 0.
+ * Floaters, replacing pymeshlab's compute_selection_by_small_disconnected_components_per_face(nbfaceratio) +
+ * compute_selection_transfer_face_to_vertex(inclusive=False) + meshing_remove_selected_vertices_and_faces: faces are
+ * connected iff they share an undirected edge {a, b}, a != b (any number of faces per edge); a component of fewer than
+ * min_faces faces is small (FloaterRemover passes int(0.005 * nF)); every vertex of a small component's face is selected
+ * and every face with a selected vertex is removed. */
+int hy3d_mesh_remove_floaters(hy3d_ctx* ctx, const float* d_verts, int64_t nV, const int32_t* d_faces, int64_t nF,
+                              int64_t min_faces, float* d_verts_out, int32_t* d_faces_out, int64_t* h_num_verts_out,
+                              int64_t* h_num_faces_out);
+/* Weld, replacing DegenerateFaceRemover's pymeshlab / trimesh round trip: every vertex is replaced by the smallest vertex id
+ * with the same three fp32 bit patterns (-0.0 taken as +0.0; a vertex with a non-finite coordinate is never merged), then
+ * a face with two equal ids is removed.  Collinear and duplicate faces are kept; there is no distance tolerance. */
+int hy3d_mesh_weld(hy3d_ctx* ctx, const float* d_verts, int64_t nV, const int32_t* d_faces, int64_t nF, float* d_verts_out,
+                   int32_t* d_faces_out, int64_t* h_num_verts_out, int64_t* h_num_faces_out);
 /* Table-independent classification for parity tests: 8-bit case per cube, [n0-1,n1-1,n2-1]. */
 int hy3d_mc_cases(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n1, int32_t n2, float level,
                   uint8_t* d_cases);
