@@ -81,10 +81,15 @@ SYMBOLS = {
     "hy3d_decode_list_values": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32,
                                           C.POINTER(C.c_float), C.POINTER(C.c_float), c_f32p]),
     "hy3d_scatter": (C.c_int, [C.c_void_p, c_i32p, c_f32p, C.c_int64, C.c_int64, c_f32p]),
+    "hy3d_scatter_window": (C.c_int, [C.c_void_p, c_i32p, c_f32p, C.c_int64, C.c_int64, C.c_int64, c_f32p]),
     "hy3d_flash_select": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Coords),
                                     c_i32p, C.c_int32, C.c_int32, C.c_int32]),
     "hy3d_decode_flash": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Coords),
                                     c_i32p, c_f32p]),
+    "hy3d_flash_select_range": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Coords),
+                                          c_i32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32]),
+    "hy3d_decode_flash_values": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Coords),
+                                           c_i32p, c_f32p]),
     "hy3d_flash_layout_bins": (C.c_int, [C.c_void_p, c_i32p, C.c_int64, C.c_int32, C.c_int32, C.c_int32, C.POINTER(Coords),
                                          C.c_int32, c_i32p, C.c_int64, c_i32p, c_i32p, C.c_int64, c_i32p, c_i32p]),
     "hy3d_flash_layout_minigrids": (C.c_int, [C.c_void_p, C.c_int32, C.c_int32, C.c_int32, c_i32p, C.c_int64, c_i32p, c_i32p,
@@ -436,6 +441,13 @@ class GeoContext:
         self._check(self.lib.hy3d_scatter(self.h, _ptr(index.contiguous()), _ptr(values.contiguous()), index.numel(), int(base),
                                           _ptr(grid)), "hy3d_scatter")
 
+    def scatter_window(self, index: torch.Tensor, values: torch.Tensor, grid: torch.Tensor, base: int):
+        """grid.flat[index[q] - base] = values[q] for the entries with base <= index[q] < base + grid.numel(), the others
+        skipped (a slab of a grid partitioned across GPUs, halo planes included)."""
+        self.sync_stream()
+        self._check(self.lib.hy3d_scatter_window(self.h, _ptr(index.contiguous()), _ptr(values.contiguous()), index.numel(),
+                                                 int(base), grid.numel(), _ptr(grid)), "hy3d_scatter_window")
+
     # ---- FlashVDM ---------------------------------------------------------------------------
     @staticmethod
     def _coords(cell=None, bmin=None, axes=None):
@@ -457,6 +469,26 @@ class GeoContext:
         c, keep = self._coords(cell, bmin, axes)
         self._check(self.lib.hy3d_flash_select(self.h, _ptr(sample_index), sample_index.numel(), dims[0], dims[1], dims[2],
                                                C.byref(c), _ptr(sample_off), n_groups, topk, int(merge)), "hy3d_flash_select")
+
+    def flash_select_range(self, sample_index: torch.Tensor, n_samples: int, dims, sample_off: torch.Tensor, n_groups: int,
+                           g0: int, g1: int, topk: int, merge: bool, cell=None, bmin=None, axes=None):
+        """``flash_select`` for groups [g0, g1) of a layout of ``n_groups``: ``sample_index`` = the layout's samples from
+        entry sample_off[g0] on, ``n_samples`` = sample_off[g1] - sample_off[g0]; ``sample_off`` = the whole layout's."""
+        self.sync_stream()
+        c, keep = self._coords(cell, bmin, axes)
+        self._check(self.lib.hy3d_flash_select_range(self.h, _ptr(sample_index), int(n_samples), dims[0], dims[1], dims[2],
+                                                     C.byref(c), _ptr(sample_off), int(n_groups), int(g0), int(g1), topk,
+                                                     int(merge)), "hy3d_flash_select_range")
+
+    def decode_flash_values(self, index: torch.Tensor, dims, tile_group: torch.Tensor, cell=None, bmin=None,
+                            axes=None) -> torch.Tensor:
+        """Compact ``decode_flash``: logits of a 128-aligned slice of a padded layout (any value at padding entries)."""
+        self.sync_stream()
+        c, keep = self._coords(cell, bmin, axes)
+        out = torch.empty(index.numel(), dtype=torch.float32, device=self.device)
+        self._check(self.lib.hy3d_decode_flash_values(self.h, _ptr(index), index.numel(), dims[0], dims[1], dims[2], C.byref(c),
+                                                      _ptr(tile_group), _ptr(out)), "hy3d_decode_flash_values")
+        return out
 
     def decode_flash(self, index: torch.Tensor, dims, tile_group: torch.Tensor, grid: torch.Tensor, cell=None, bmin=None,
                      axes=None):

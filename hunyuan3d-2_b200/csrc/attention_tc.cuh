@@ -53,6 +53,7 @@ struct AttnTC {
   const int* tile_group; // per q-tile KV group or null
   const int* group_ntok; // valid tokens per group or null
   int Pb, H, nkv, ntok;  // nkv = tiles per (group, head); ntok = valid tokens when group_ntok == null
+  int group_base;        // K / V / group_ntok hold groups group_base, group_base + 1, ... (tile_group values are absolute)
   int split_out;         // O written as [hi | lo | hi] over 3H k-blocks (operand of a 3-term split GEMM)
   int share_kv;          // 1: streams = two query tiles of one head sharing every K/V tile; 0: two heads of one query tile
   // K / V gathered from several GPUs (sequence-parallel latent transformer): tile j of head h lives in chunk j / kv_tpr at
@@ -161,7 +162,7 @@ __device__ __forceinline__ void attn_producer(const AttnTC& g, const AttnBars& B
       __syncwarp();
     }
     qph ^= 1;
-    const int grp = g.tile_group ? g.tile_group[it.qt] : 0;
+    const int grp = g.tile_group ? g.tile_group[it.qt] - g.group_base : 0;
     const int tpr = g.kv_tpr ? g.kv_tpr : nkv;
     const size_t head_off = ((size_t)grp * g.H + it.h) * tpr * TILE_BYTES;
     auto tile = [&](const uint8_t* base, int j) {
@@ -332,7 +333,7 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
     for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
       const AttnItem wi = attn_item(g, item, a);
       const int qt = wi.qt, h = wi.h;
-      const int ntok = g.group_ntok ? g.group_ntok[g.tile_group ? g.tile_group[qt] : 0] : g.ntok;
+      const int ntok = g.group_ntok ? g.group_ntok[g.tile_group ? g.tile_group[qt] - g.group_base : 0] : g.ntok;
       uint64_t l2 = 0ull;                                // packed (even columns, odd columns) row sums: one FADD2 per pair
       const float cshift = g.head_shift ? g.head_shift[h] : 0.f;       // 0 unless the head's measured score bound exceeds 15.9
       const uint64_t cshift2 = pack_f2(cshift, cshift);
@@ -514,7 +515,7 @@ __global__ void __launch_bounds__(ATT_THREADS, 1) k_attn_tc(AttnTC g) {
     for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
       const AttnItem wi = attn_item(g, item, a);
       const int qt = wi.qt, h = wi.h;
-      const int ntok = g.group_ntok ? g.group_ntok[g.tile_group ? g.tile_group[qt] : 0] : g.ntok;
+      const int ntok = g.group_ntok ? g.group_ntok[g.tile_group ? g.tile_group[qt] - g.group_base : 0] : g.ntok;
       float m = -INFINITY;
       uint64_t l2 = 0ull;                               // packed (even, odd column) partial row sums of this half
       for (int j = 0; j < nkv; ++j) {

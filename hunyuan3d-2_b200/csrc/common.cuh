@@ -73,6 +73,7 @@ struct KVState {
 struct KVSelState {
   bool ready = false;
   int G = 0, nkv = 0;                 // groups, 128-token tiles per (group, head)
+  int g0 = 0;                         // layout group of local group 0 (hy3d_flash_select_range)
   DevBuf ktile, vtile;                // [G][H][nkv][16 KB]
   DevBuf ntok;                        // int [G] valid tokens per group
   DevBuf sel;                         // int [G][H][T] (mean) or [G][Mpad] (merge) selected token ids

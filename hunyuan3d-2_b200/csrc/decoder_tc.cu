@@ -1344,7 +1344,7 @@ static int decode_tc_impl(hy3d_ctx* ctx, const QuerySource& src_in, long long n,
       a.Q = ta; a.O = tq; a.Pb = Pb; a.H = H;
       if (d_tile_group) {
         a.K = ctx->kvsel.ktile.as<uint8_t>(); a.V = ctx->kvsel.vtile.as<uint8_t>(); a.nkv = ctx->kvsel.nkv;
-        a.tile_group = d_tile_group + p0 / 128; a.group_ntok = ctx->kvsel.ntok.as<int>();
+        a.tile_group = d_tile_group + p0 / 128; a.group_ntok = ctx->kvsel.ntok.as<int>(); a.group_base = ctx->kvsel.g0;
       } else {
         a.K = ctx->kv.ktile.as<uint8_t>(); a.V = ctx->kv.vtile.as<uint8_t>(); a.nkv = ctx->kv.Mpad / 128; a.ntok = ctx->kv.M;
       }

@@ -18,10 +18,11 @@ namespace {
 
 constexpr int TILE_BYTES = 16384;
 
-// qbar[g][c] = mean over samples of group g of qs[s][c]
+// qbar[g][c] = mean over samples of group g of qs[s][c].  off = the sample offsets of the selected groups; qs row 0 is the
+// sample at off[0] (a range of groups starting past group 0 has its samples' q rows only)
 __global__ void k_group_mean(const float* __restrict__ qs, const int* __restrict__ off, int W, float* __restrict__ qbar) {
   const int g = blockIdx.x;
-  const int s0 = off[g], s1 = off[g + 1];
+  const int s0 = off[g] - off[0], s1 = off[g + 1] - off[0];
   for (int c = threadIdx.x; c < W; c += blockDim.x) {
     float acc = 0.f;
     for (int s = s0; s < s1; ++s) acc += qs[(size_t)s * W + c];
@@ -132,12 +133,12 @@ __global__ void __launch_bounds__(1024) k_sim_topk(const float* __restrict__ qba
 __global__ void __launch_bounds__(256) k_merge_flags(const float* __restrict__ qs, const int* __restrict__ off, int G, int H, int M,
                                                      const float* __restrict__ k32, float thresh, uint32_t* __restrict__ mask,
                                                      int mwords) {
-  const int s = blockIdx.x;
-  if (s >= off[G]) return;
+  const int s = blockIdx.x, s0 = off[0];        // qs row s = sample s0 + s (see k_group_mean)
+  if (s >= off[G] - s0) return;
   __shared__ int gsh;
   __shared__ float qv[64];
   __shared__ float red[8];
-  if (threadIdx.x == 0) { int g = 0; while (g + 1 < G && off[g + 1] <= s) ++g; gsh = g; }
+  if (threadIdx.x == 0) { int g = 0; while (g + 1 < G && off[g + 1] - s0 <= s) ++g; gsh = g; }
   constexpr int PER = 16;                      // tokens per thread (M <= 4096)
   float acc[PER];
 #pragma unroll
@@ -275,7 +276,19 @@ extern "C" {
 
 int hy3d_flash_select(hy3d_ctx* ctx, const int32_t* d_sample_index, int64_t n_samples, int32_t n0, int32_t n1, int32_t n2,
                       const hy3d_coords* coords, const int32_t* d_sample_off, int32_t G, int32_t topk, int32_t merge_mode) {
-  if (!ctx || !d_sample_index || !coords || !d_sample_off || G <= 0 || n_samples <= 0) return HY3D_ERR_ARG;
+  return hy3d_flash_select_range(ctx, d_sample_index, n_samples, n0, n1, n2, coords, d_sample_off, G, 0, G, topk, merge_mode);
+}
+
+// groups [g0, g1) of a layout: d_sample_index = the layout's sample list from entry d_sample_off[g0] on, d_sample_off = the
+// whole layout's offsets; the selection is stored under the local group ids 0 .. g1-g0-1 and hy3d_decode_flash(_values)
+// subtracts g0 from every tile's group
+int hy3d_flash_select_range(hy3d_ctx* ctx, const int32_t* d_sample_index, int64_t n_samples, int32_t n0, int32_t n1, int32_t n2,
+                            const hy3d_coords* coords, const int32_t* d_sample_off, int32_t G_all, int32_t g0, int32_t g1,
+                            int32_t topk, int32_t merge_mode) {
+  if (!ctx || !d_sample_index || !coords || !d_sample_off || G_all <= 0 || n_samples <= 0) return HY3D_ERR_ARG;
+  if (g0 < 0 || g1 <= g0 || g1 > G_all) return hy3d_fail(ctx, HY3D_ERR_ARG, "group range [%d, %d) outside [0, %d)", g0, g1, G_all);
+  const int G = g1 - g0;
+  d_sample_off += g0;
   if (!ctx->w.set || !ctx->kv.ready) return hy3d_fail(ctx, HY3D_ERR_STATE, "weights / K,V not prepared");
   if (ctx->precision != HY3D_PRECISION_FP16_TC) return hy3d_fail(ctx, HY3D_ERR_UNSUPPORTED, "FlashVDM runs on the tcgen05 path only");
   HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
@@ -329,6 +342,7 @@ int hy3d_flash_select(hy3d_ctx* ctx, const int32_t* d_sample_index, int64_t n_sa
                                                                          ks.ntok.as<int>(), ks.ktile.as<uint8_t>(), ks.vtile.as<uint8_t>(), total);
   HY3D_LAUNCH_CHECK(ctx);
   ks.G = G;
+  ks.g0 = g0;
   ks.ready = true;
   return HY3D_OK;
 }
@@ -343,6 +357,18 @@ int hy3d_decode_flash(hy3d_ctx* ctx, const int32_t* d_index, int64_t n, int32_t 
   QuerySource src;
   if (int rc = make_source(ctx, coords, d_index, n0, n1, n2, src)) return rc;
   return hy3d_decode_tc_groups(ctx, src, n, d_grid, 1, d_tile_group);
+}
+
+int hy3d_decode_flash_values(hy3d_ctx* ctx, const int32_t* d_index, int64_t n, int32_t n0, int32_t n1, int32_t n2,
+                             const hy3d_coords* coords, const int32_t* d_tile_group, float* d_values) {
+  if (!ctx || n < 0 || !coords) return HY3D_ERR_ARG;
+  if (n == 0) return HY3D_OK;
+  if (!d_index || !d_tile_group || !d_values || (n % 128) != 0) return hy3d_fail(ctx, HY3D_ERR_ARG, "padded list must be a multiple of 128");
+  if (ctx->precision != HY3D_PRECISION_FP16_TC) return hy3d_fail(ctx, HY3D_ERR_UNSUPPORTED, "FlashVDM runs on the tcgen05 path only");
+  HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
+  QuerySource src;
+  if (int rc = make_source(ctx, coords, d_index, n0, n1, n2, src)) return rc;
+  return hy3d_decode_tc_groups(ctx, src, n, d_values, 0, d_tile_group);
 }
 
 // selected token ids of the last hy3d_flash_select (selection-parity tests): mean mode int32 [G,H,T]

@@ -186,12 +186,13 @@ __global__ void k_fill_f32(float* __restrict__ p, long long n, float v) {
   for (; t < n; t += stride) p[t] = v;
 }
 
+// entries outside the window [base, base + len) of the whole grid (padding -1 included) are skipped
 __global__ void k_scatter_f32(const int32_t* __restrict__ index, const float* __restrict__ vals, long long n, long long base,
-                              float* __restrict__ grid) {
+                              long long len, float* __restrict__ grid) {
   long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
   if (t >= n) return;
   int i = index[t];
-  if (i < 0) return;
+  if (i < base || i - base >= len) return;
   float v = vals[t];
   if (v == HY3D_SENTINEL) v = __int_as_float(0x7fc00000);    // a logit equal to the sentinel is "unvisited" downstream (volume_decoders.py:275)
   grid[i - base] = v;
@@ -275,7 +276,18 @@ int hy3d_scatter(hy3d_ctx* ctx, const int32_t* d_index, const float* d_values, i
   if (n == 0) return HY3D_OK;
   HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
   HY3D_PROF(ctx, FAM_OCTREE);
-  k_scatter_f32<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(d_index, d_values, n, base, d_grid);
+  k_scatter_f32<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(d_index, d_values, n, base, LLONG_MAX, d_grid);
+  HY3D_LAUNCH_CHECK(ctx);
+  return HY3D_OK;
+}
+
+int hy3d_scatter_window(hy3d_ctx* ctx, const int32_t* d_index, const float* d_values, int64_t n, int64_t base, int64_t len,
+                        float* d_grid) {
+  if (!ctx || n < 0 || base < 0 || len < 0 || (n > 0 && len > 0 && (!d_index || !d_values || !d_grid))) return HY3D_ERR_ARG;
+  if (n == 0 || len == 0) return HY3D_OK;
+  HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
+  HY3D_PROF(ctx, FAM_OCTREE);
+  k_scatter_f32<<<(unsigned)ceil_div64(n, 256), 256, 0, ctx->stream>>>(d_index, d_values, n, base, len, d_grid);
   HY3D_LAUNCH_CHECK(ctx);
   return HY3D_OK;
 }

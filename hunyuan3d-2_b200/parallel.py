@@ -19,13 +19,16 @@ gloo and a fake field (tests/test_parallel_gloo.py).
 """
 from __future__ import annotations
 
-from typing import Callable, List, Optional, Tuple
+import bisect
+import itertools
+from typing import Callable, List, Optional, Sequence, Tuple
 
 import numpy as np
 import torch
 import torch.distributed as dist
 
-from .volume_decoders import (SENTINEL, axis_tables, bind, hierarchy_levels, normalize_bounds, refine_level)
+from .volume_decoders import (NAN, SENTINEL, axis_tables, bind, flash_levels, flash_topk_budget, hierarchy_levels, normalize_bounds,
+                              refine_level)
 
 
 def slab_planes(n_planes: int, rank: int, world: int) -> Tuple[int, int]:
@@ -348,7 +351,23 @@ def plane_cuts(index: torch.Tensor, n: int, world: int, halo: int = MC_HALO):
     return planes, at[: world + 1], at[world + 1:]
 
 
-class ShardedHierarchicalVolumeDecoding:
+class _StageTimeline:
+    """Diagnostics of the sharded sparse decoders: with ``self.timeline`` a dict, ``_tick(name)`` adds the wall time since the
+    previous tick to stage ``name`` (ms, accumulated; synchronises the device; tools/gpu_hier_timeline.py)."""
+    timeline = None
+
+    def _tick(self, name, dev):
+        if self.timeline is None:
+            return
+        import time
+        torch.cuda.synchronize(dev)
+        now = time.perf_counter()
+        if getattr(self, "_t_last", None) is not None and name:
+            self.timeline[name] = self.timeline.get(name, 0.0) + (now - self._t_last) * 1e3
+        self._t_last = now
+
+
+class ShardedHierarchicalVolumeDecoding(_StageTimeline):
     """HierarchicalVolumeDecoding (reference :185-277, patched coordinates) over a process group.
 
     Coarse levels: every rank evaluates its share (level 0: an axis-0 slab; refined levels: an equal contiguous range
@@ -365,16 +384,6 @@ class ShardedHierarchicalVolumeDecoding:
         self.group = group
         self.keep_sharded = keep_sharded
         self.timeline = {} if timeline else None      # diagnostics: stage -> accumulated ms (synchronising; tools/gpu_hier_timeline.py)
-
-    def _tick(self, name, dev):
-        if self.timeline is None:
-            return
-        import time
-        torch.cuda.synchronize(dev)
-        now = time.perf_counter()
-        if getattr(self, "_t_last", None) is not None and name:
-            self.timeline[name] = self.timeline.get(name, 0.0) + (now - self._t_last) * 1e3
-        self._t_last = now
 
     @torch.no_grad()
     def __call__(self, latents, geo_decoder, bounds=1.01, num_chunks=10000, mc_level=0.0, octree_resolution=None,
@@ -453,6 +462,151 @@ class ShardedHierarchicalVolumeDecoding:
                 self._tick(f"level {n}^3 decode + all_gather + scatter", latents.device)
             if not sharded_last:
                 ctx.sentinel_to_nan(grid, SENTINEL)
+            outs.append(grid)
+            self.last_stats.append({"levels": levels, "queries": queries, "rank_queries": mine})
+        if sharded_last:
+            N = levels[-1] + 1
+            return SlabGrid(outs, plane0s, owns, (N, N, N), True, self.group, latents.dtype)
+        return torch.stack(outs, 0).to(latents.dtype)
+
+
+def flash_partition(tiles_per_group: Sequence[int], world: int) -> List[Tuple[int, int, int, int]]:
+    """Split the tiles of a group-ordered, 128-padded FlashVDM list into ``world`` contiguous runs whose tile counts differ
+    by at most one (decoder work balanced to within one tile).  Returns per rank (t0, t1, g0, g1): tiles [t0, t1) and the
+    groups [g0, g1) they use, from the group of the first tile to the group of the last.  A group cut by a boundary is
+    selected by both neighbours; a rank without tiles gets (t0, t0, 0, 0)."""
+    ends = list(itertools.accumulate(int(t) for t in tiles_per_group))
+    total = ends[-1] if ends else 0
+    parts = []
+    for r in range(world):
+        t0, t1 = list_range(total, r, world)
+        if t1 == t0:
+            parts.append((t0, t1, 0, 0))
+        else:                                   # group of tile t = the first group whose tiles end past t
+            parts.append((t0, t1, bisect.bisect_right(ends, t0), bisect.bisect_right(ends, t1 - 1) + 1))
+    return parts
+
+
+def flash_minigrid_sizes(N: int, mini_grid_num: int, stride: int = 100) -> Tuple[List[int], List[int]]:
+    """Host image of the level-0 layout hy3d_flash_layout_minigrids writes: (queries per mini-grid, sample offsets [G+1]).
+    Every mini-grid holds s^3 queries (s = N / mini_grid_num) padded to whole tiles and ceil(s^3 / stride) samples."""
+    m = int(mini_grid_num)
+    s3 = (int(N) // m) ** 3
+    nsamp = -(-s3 // int(stride))
+    return [s3] * m ** 3, [g * nsamp for g in range(m ** 3 + 1)]
+
+
+def _tile_queries(counts: Sequence[int], t0: int, t1: int) -> int:
+    """Real (non-padding) queries in tiles [t0, t1) of a padded list whose groups hold ``counts`` queries."""
+    q, a = 0, 0
+    for c in counts:
+        k = -(-int(c) // 128)
+        lo, hi = max(t0, a), min(t1, a + k)
+        if hi > lo:
+            q += min(c, 128 * (hi - a)) - min(c, 128 * (lo - a))
+        a += k
+    return q
+
+
+class ShardedFlashVDMVolumeDecoding(_StageTimeline):
+    """FlashVDMVolumeDecoding (reference volume_decoders.py:280-435) over a process group; same call signature, and the
+    same grid bit for bit (NaNs included).
+
+    Every rank holds the same K/V, refined active list and group layout (level 0: mini_grid_num^3 mini-grids; refined
+    levels: 6^3 spatial bins), all cheap and deterministic.  The padded list's tiles are split into contiguous runs of
+    near-equal length (``flash_partition``); each rank selects the K/V tokens of the groups its run touches (a group cut
+    by a boundary is selected by both neighbours, identically) and decodes its run into compact values, which are
+    all-gathered.  Level 0 and intermediate levels are then scattered into the whole grid on every rank.  The last level
+    (``keep_sharded``, default, more than one level): each rank scatters into its plane-aligned slab (``plane_cuts``) plus
+    the two-plane marching-cubes halo only and a ``SlabGrid`` is returned — no full-resolution grid on any rank.
+    Otherwise the ordinary latents.dtype tensor is returned on every rank.  A refined level adds one host read-back (the
+    216 bin counts and sample offsets) to what the single-GPU decoder synchronises on.
+
+    ``last_stats[b]``: levels, queries (as FlashVDMVolumeDecoding), rank_queries (real queries this rank decoded)."""
+
+    def __init__(self, topk_mode='mean', group=None, keep_sharded: bool = True, timeline: bool = False):
+        if topk_mode not in ['mean', 'merge']:
+            raise ValueError(f'Unsupported topk_mode {topk_mode}, available: {["mean", "merge"]}')
+        self.topk_mode = topk_mode
+        self.group = group
+        self.keep_sharded = keep_sharded
+        self.timeline = {} if timeline else None
+
+    def _level(self, ctx, dims, layout, soff_h, counts, topk, merge, coords):
+        """Select + decode this rank's run of a level's layout; -> (values of the whole padded list, this rank's queries)."""
+        pidx, tile_group, sidx, soff = layout
+        rank, world = dist.get_rank(self.group), dist.get_world_size(self.group)
+        parts = flash_partition([-(-c // 128) for c in counts], world)
+        t0, t1, g0, g1 = parts[rank]
+        vals = torch.empty(0, dtype=torch.float32, device=pidx.device)
+        if t1 > t0:
+            ctx.flash_select_range(sidx[soff_h[g0]:], soff_h[g1] - soff_h[g0], dims, soff, len(counts), g0, g1, topk, merge, **coords)
+            vals = ctx.decode_flash_values(pidx[t0 * 128: t1 * 128], dims, tile_group[t0:t1], **coords)
+        vals = all_gather_ranges(vals, [(b - a) * 128 for a, b, _, _ in parts], self.group)
+        return vals, _tile_queries(counts, t0, t1)
+
+    @torch.no_grad()
+    def __call__(self, latents, geo_decoder, bounds=1.01, num_chunks=10000, mc_level=0.0, octree_resolution=None,
+                 min_resolution=63, mini_grid_num=4, enable_pbar=True, **kwargs):
+        dev = latents.device
+        self._tick(None, dev)
+        ctx = bind(latents, geo_decoder)
+        levels = flash_levels(octree_resolution, min_resolution, mini_grid_num)
+        b6 = normalize_bounds(bounds)
+        bbox_min, bbox_size = b6[:3], b6[3:] - b6[:3]
+        bmin32 = bbox_min.astype(np.float32)
+        merge = self.topk_mode == 'merge'
+        rank, world = dist.get_rank(self.group), dist.get_world_size(self.group)
+        sharded_last = self.keep_sharded and len(levels) > 1 and levels[-1] + 1 >= MC_HALO * world
+        T = flash_topk_budget(latents.shape[1])
+        outs, plane0s, owns = [], [], []
+        self.last_stats = []
+        for b in range(latents.shape[0]):
+            ctx.prepare_kv(latents[b])
+            self._tick("kv_prepare (replicated)", dev)
+            # ---- level 0: mini-grids; sizes known on the host (level 0 is 'mean' in both modes, as in FlashVDMVolumeDecoding)
+            N0 = levels[0] + 1
+            layout = ctx.flash_layout_minigrids(N0, mini_grid_num, 100)
+            counts, soff_h = flash_minigrid_sizes(N0, mini_grid_num, 100)
+            self._tick("level0 layout (replicated)", dev)
+            vals, mine0 = self._level(ctx, (N0, N0, N0), layout, soff_h, counts, T, False, dict(axes=axis_tables(bounds, levels[0])))
+            grid = torch.empty((N0, N0, N0), dtype=torch.float32, device=dev)
+            ctx.scatter(layout[0][: vals.numel()], vals, grid)
+            self._tick("level0 select + decode + all_gather + scatter", dev)
+            queries, mine = [N0 ** 3], [mine0]
+            # ---- refined levels: 6^3 spatial bins of the active queries
+            for r in levels[1:]:
+                n = r + 1
+                last = r == levels[-1]
+                index = refine_level(ctx, grid, mc_level, last=last, nf=n)
+                self._tick(f"refine -> {n}^3 (replicated)", dev)
+                cell = (bbox_size / r).astype(np.float32)
+                nq = int(index.numel())
+                queries.append(nq)
+                if nq:                  # nq is the same on every rank: an empty level is skipped by all alike
+                    *layout, counts_d = ctx.flash_layout_bins(index, (n, n, n), cell, bmin32, 30 if merge else 50, with_counts=True)
+                    meta = torch.cat([counts_d, layout[3]]).tolist()          # one small read-back: 216 counts + 217 offsets
+                    self._tick(f"level {n}^3 layout + count read-back (replicated)", dev)
+                    vals, m = self._level(ctx, (n, n, n), layout, meta[216:], meta[:216], T, merge, dict(cell=cell, bmin=bmin32))
+                    self._tick(f"level {n}^3 select + decode + all_gather", dev)
+                mine.append(m if nq else 0)
+                if last and sharded_last:
+                    planes, _, _ = plane_cuts(index, n, world)
+                    plane0, own = planes[rank], planes[rank + 1] - planes[rank]
+                    slab = torch.empty((min(planes[rank + 1] + MC_HALO, n) - plane0, n, n), dtype=torch.float32, device=dev)
+                    ctx.fill(slab, NAN)
+                    if nq:
+                        ctx.scatter_window(layout[0][: vals.numel()], vals, slab, plane0 * n * n)
+                    grid = slab
+                    plane0s.append(plane0); owns.append(own)
+                    self._tick("last level scatter (own slab)", dev)
+                    break
+                nxt = torch.empty((n, n, n), dtype=torch.float32, device=dev)
+                ctx.fill(nxt, NAN if last else SENTINEL)
+                if nq:
+                    ctx.scatter(layout[0][: vals.numel()], vals, nxt)
+                grid = nxt
+                self._tick(f"level {n}^3 scatter", dev)
             outs.append(grid)
             self.last_stats.append({"levels": levels, "queries": queries, "rank_queries": mine})
         if sharded_last:

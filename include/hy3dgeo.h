@@ -147,6 +147,11 @@ int hy3d_decode_list_values(hy3d_ctx* ctx, const int32_t* d_index, int64_t n, in
  * `base` = flat index of d_grid[0] in the whole grid (0, or the first voxel of a slab kept by one GPU);
  * every non-negative d_index[q] must be >= base.  Entries with d_index[q] < 0 are skipped. */
 int hy3d_scatter(hy3d_ctx* ctx, const int32_t* d_index, const float* d_values, int64_t n, int64_t base, float* d_grid);
+/* Windowed form of hy3d_scatter for a slab of a grid that is partitioned across GPUs: d_grid holds the flat indices
+ * [base, base + len) of the whole grid; only the entries with base <= d_index[q] < base + len are written (as
+ * d_grid[d_index[q] - base], a logit equal to the -10000 sentinel as NaN, like hy3d_scatter), all others are skipped. */
+int hy3d_scatter_window(hy3d_ctx* ctx, const int32_t* d_index, const float* d_values, int64_t n, int64_t base, int64_t len,
+                        float* d_grid);
 
 /* ---- FlashVDM: replaces FlashVDMVolumeDecoding's decoder calls (volume_decoders.py:343-371,
  * 398-431) and the processors of attention_processors.py:35-96 ------------------------------ */
@@ -169,6 +174,21 @@ int hy3d_flash_select(hy3d_ctx* ctx, const int32_t* d_sample_index, int64_t n_sa
  * tile's group (d_tile_group: DEVICE int32 [n/128]); logits scattered to d_grid[d_index[q]]. */
 int hy3d_decode_flash(hy3d_ctx* ctx, const int32_t* d_index, int64_t n, int32_t n0, int32_t n1, int32_t n2,
                       const hy3d_coords* coords, const int32_t* d_tile_group, float* d_grid);
+/* Multi-GPU forms (no reference counterpart: the reference is single-device; SURVEY §8e).  One GPU selects and decodes a
+ * contiguous run of tiles of a layout; the groups its tiles use are [g0, g1).
+ * hy3d_flash_select_range: hy3d_flash_select restricted to groups [g0, g1) of a layout of G groups.  d_sample_off is the
+ * whole layout's DEVICE int32 [G+1]; d_sample_index points at that layout's sample d_sample_off[g0] and n_samples =
+ * d_sample_off[g1] - d_sample_off[g0] (known to the caller: no host synchronisation).  Each group's selection is exactly
+ * the one hy3d_flash_select makes for it; it is stored under the local ids 0 .. g1-g0-1, and until the next selection
+ * hy3d_decode_flash and hy3d_decode_flash_values take a tile's K/V from local group d_tile_group[t] - g0
+ * (hy3d_flash_select = the range [0, G)).  A bad range returns HY3D_ERR_ARG.
+ * hy3d_decode_flash_values: hy3d_decode_flash with a compact result, d_values[q] = logit of d_index[q] (any value at
+ * padding entries); d_index / d_tile_group may be a 128-aligned slice of a layout. */
+int hy3d_flash_select_range(hy3d_ctx* ctx, const int32_t* d_sample_index, int64_t n_samples, int32_t n0, int32_t n1, int32_t n2,
+                            const hy3d_coords* coords, const int32_t* d_sample_off, int32_t G, int32_t g0, int32_t g1,
+                            int32_t topk, int32_t merge_mode);
+int hy3d_decode_flash_values(hy3d_ctx* ctx, const int32_t* d_index, int64_t n, int32_t n0, int32_t n1, int32_t n2,
+                             const hy3d_coords* coords, const int32_t* d_tile_group, float* d_values);
 /* Query layout of a refined FlashVDM level, all on the device (no host synchronisation): replaces
  * volume_decoders.py:394-412 -- bin id of every active query (float32 op for op: floor((p - min) /
  * (max - min) * (6 - 0.001)) per axis, 6^3 = 216 bins, ids clamped to [0, 215]), STABLE sort by bin,
