@@ -3,7 +3,7 @@
 Drop-in replacements for the reference's ``volume_decoder`` / ``surface_extractor``
 plugin slots (reference hy3dgen/shapegen/models/autoencoders/model.py:92-110)
 and for the ``FloaterRemover`` / ``DegenerateFaceRemover`` mesh filters
-(reference hy3dgen/shapegen/postprocessors.py), backed by hand-written CUDA kernels behind the C-ABI declared in
+(reference hy3dgen/shapegen/postprocessors.py; ``FaceReducer`` is ``hy3dgeo.postprocessors.FaceReducer``), backed by hand-written CUDA kernels behind the C-ABI declared in
 ``include/hy3dgeo.h``.  There is no CPU fallback: every compute entry point
 raises if ``libhy3dgeo.so`` is missing.
 """

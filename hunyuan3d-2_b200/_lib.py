@@ -117,6 +117,8 @@ SYMBOLS = {
                                             C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "hy3d_mesh_weld": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, c_f32p, c_i32p,
                                  C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
+    "hy3d_mesh_decimate": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int64, c_f32p, c_i32p,
+                                     C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_int32)]),
     "hy3d_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "hy3d_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "hy3d_debug_watchdog": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
@@ -614,7 +616,7 @@ class GeoContext:
                                              _ptr(vo), _ptr(fo), C.byref(nv), C.byref(nf)), "hy3d_mesh_clean")
         return vo[: nv.value], fo[: nf.value]
 
-    def _mesh_filter(self, name, verts, faces, *args):
+    def _mesh_filter(self, name, verts, faces, *args, extra=()):
         self.sync_stream()
         verts = verts.detach().to(device=self.device, dtype=torch.float32).contiguous()
         faces = faces.detach().to(device=self.device, dtype=torch.int32).contiguous()
@@ -623,7 +625,7 @@ class GeoContext:
         vo, fo = torch.empty_like(verts), torch.empty_like(faces)
         nv, nf = C.c_int64(), C.c_int64()
         self._check(getattr(self.lib, name)(self.h, _ptr(verts), verts.shape[0], _ptr(faces), faces.shape[0], *args,
-                                            _ptr(vo), _ptr(fo), C.byref(nv), C.byref(nf)), name)
+                                            _ptr(vo), _ptr(fo), C.byref(nv), C.byref(nf), *extra), name)
         return vo[: nv.value], fo[: nf.value]
 
     def mesh_remove_floaters(self, verts: torch.Tensor, faces: torch.Tensor, min_faces: int):
@@ -635,6 +637,13 @@ class GeoContext:
         """Device tensors -> the mesh with bit-equal finite vertices merged into the smallest id, faces that collapse
         removed, unreferenced vertices dropped, order kept (hy3dgeo.h)."""
         return self._mesh_filter("hy3d_mesh_weld", verts, faces)
+
+    def mesh_decimate(self, verts: torch.Tensor, faces: torch.Tensor, max_faces: int):
+        """Device tensors -> (verts, faces, rounds): quadric edge-collapse decimation to ``max_faces`` faces (``max_faces - 1``
+        or ``max_faces`` unless no valid collapse is left); the mesh as given when it has no more faces (hy3dgeo.h)."""
+        rounds = C.c_int32()
+        vo, fo = self._mesh_filter("hy3d_mesh_decimate", verts, faces, int(max_faces), extra=(C.byref(rounds),))
+        return vo, fo, rounds.value
 
     def mc_cases(self, grid: torch.Tensor, level: float) -> torch.Tensor:
         self.sync_stream()

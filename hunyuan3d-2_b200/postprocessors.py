@@ -1,18 +1,20 @@
-"""Mesh post-processing on the GPU — ``FloaterRemover`` and ``DegenerateFaceRemover`` of the reference's
+"""Mesh post-processing on the GPU — ``FloaterRemover``, ``DegenerateFaceRemover`` and ``FaceReducer`` of the reference's
 ``hy3dgen/shapegen/postprocessors.py``, which every Hunyuan3D-2 front end runs on the mesh ``latents2mesh`` returns::
 
     mesh = FloaterRemover()(mesh)
     mesh = DegenerateFaceRemover()(mesh)
+    mesh = FaceReducer()(mesh)          # max_facenum=40000
 
-The reference builds both on pymeshlab (CPU).  Here they are ``hy3d_mesh_remove_floaters`` / ``hy3d_mesh_weld`` of
-``libhy3dgeo.so``; the contract they meet bit for bit is ``oracle/postprocess.py`` (DESIGN.md §2: parity with pymeshlab is
-unpinned).  ``FaceReducer`` (quadric edge-collapse decimation) is not provided: keep pymeshlab's.
+The reference builds all three on pymeshlab (CPU).  Here they are ``hy3d_mesh_remove_floaters`` / ``hy3d_mesh_weld`` /
+``hy3d_mesh_decimate`` of ``libhy3dgeo.so``; the contracts they meet bit for bit are ``oracle/postprocess.py`` and
+``oracle/decimate.py`` (DESIGN.md §2: parity with pymeshlab is unpinned).  ``FaceReducer`` keeps boundaries exactly,
+never lets a face flip, and collapses edges in rounds of independent collapses instead of one heap.
 
 Each class takes a ``Latent2MeshOutput`` (returns a new one holding float32 / int32 numpy arrays) or a ``trimesh.Trimesh``
 (returns ``trimesh.Trimesh(..., process=False)``); the input is never modified.  Positions are processed in float32.
 Anything else — a path, a pymeshlab ``MeshSet`` — raises ``TypeError``.  There is no CPU path: without a CUDA device the
-call raises ``RuntimeError``.  ``run_device(verts, faces)`` works on CUDA tensors, so the two filters chain without the mesh
-crossing PCIe in between.
+call raises ``RuntimeError``.  ``run_device(verts, faces)`` works on CUDA tensors, so the three filters chain without the
+mesh crossing PCIe in between.
 """
 from __future__ import annotations
 
@@ -82,3 +84,26 @@ class DegenerateFaceRemover:
         """CUDA tensors (verts float32 [V, 3], faces int32 [F, 3]) -> the welded mesh as device tensors."""
         _check_device_mesh(verts, faces)
         return get_context(verts.device).mesh_weld(verts, faces)
+
+
+class FaceReducer:
+    """Quadric edge-collapse decimation to ``max_facenum`` faces (the result has ``max_facenum - 1`` or ``max_facenum``
+    faces, more only when no valid collapse is left); a mesh with no more than ``max_facenum`` faces is returned as given.
+    Boundary and non-manifold vertices never move, collapses that would flip a face or change the topology are refused,
+    and the order of the surviving vertices and faces is kept (hy3dgeo.h: hy3d_mesh_decimate)."""
+
+    @utils.synchronize_timer('FaceReducer')
+    def __call__(self, mesh, max_facenum: int = 40000):
+        _check_max_facenum(max_facenum)
+        return _apply(mesh, lambda v, f: self.run_device(v, f, max_facenum))
+
+    def run_device(self, verts: torch.Tensor, faces: torch.Tensor, max_facenum: int = 40000):
+        """CUDA tensors (verts float32 [V, 3], faces int32 [F, 3]) -> the decimated mesh as device tensors."""
+        _check_device_mesh(verts, faces)
+        _check_max_facenum(max_facenum)
+        return get_context(verts.device).mesh_decimate(verts, faces, int(max_facenum))[:2]
+
+
+def _check_max_facenum(max_facenum):
+    if int(max_facenum) < 1:
+        raise ValueError(f"max_facenum must be >= 1, got {max_facenum}")

@@ -292,6 +292,24 @@ int hy3d_mesh_remove_floaters(hy3d_ctx* ctx, const float* d_verts, int64_t nV, c
  * a face with two equal ids is removed.  Collinear and duplicate faces are kept; there is no distance tolerance. */
 int hy3d_mesh_weld(hy3d_ctx* ctx, const float* d_verts, int64_t nV, const int32_t* d_faces, int64_t nF, float* d_verts_out,
                    int32_t* d_faces_out, int64_t* h_num_verts_out, int64_t* h_num_faces_out);
+/* Quadric edge-collapse decimation, replacing FaceReducer's pymeshlab meshing_decimation_quadric_edge_collapse(
+ * targetfacenum=max_faces, qualitythr=1.0, preserveboundary=True, boundaryweight=3, preservenormal=True,
+ * preservetopology=True, autoclean=True); contract oracle/decimate.py, parity with pymeshlab unpinned.  nF <= max_faces:
+ * the mesh is copied as given.  Otherwise rounds of independent collapses, each on the compacted mesh of the previous one:
+ * vertices on boundary or non-manifold edges, without one closed fan, in a face with a repeated id or non-finite never move;
+ * a candidate edge (a, b) has exactly two oppositely oriented faces (a, b, c) and (b, a, d), free ends, common neighbours
+ * exactly {c, d}, deg(a) + deg(b) - 4 >= 3 and deg(c), deg(d) >= 4; a takes the float32-rounded cheapest of the minimiser of
+ * Qa + Qb (unit plane quadrics of the input, |det| >= 1e-12), pa, pb and the midpoint; the collapse is invalid if a face
+ * of the two stars would get n_old . n_new <= 0; cost = max(pQp, 1e-15) / min(worst new face quality, 1).  Edges ranked
+ * by (cost, edge id) are selected when their rank is the smallest over both ends and their neighbours, and at most
+ * ceil((F - max_faces) / 2) of them apply, so the result has max_faces - 1 or max_faces faces unless a round finds no
+ * valid collapse (the mesh is then returned with more faces).  Same buffers, int32 rules and output order as
+ * hy3d_mesh_weld; max_faces < 1 and a face index outside [0, nV) return HY3D_ERR_ARG.  *h_rounds = rounds that applied
+ * collapses.  One host synchronisation per round (the new counts and the error flag); the final copies into the output
+ * buffers are enqueued on the context's stream after the last one. */
+int hy3d_mesh_decimate(hy3d_ctx* ctx, const float* d_verts, int64_t nV, const int32_t* d_faces, int64_t nF, int64_t max_faces,
+                       float* d_verts_out, int32_t* d_faces_out, int64_t* h_num_verts_out, int64_t* h_num_faces_out,
+                       int32_t* h_rounds);
 /* Table-independent classification for parity tests: 8-bit case per cube, [n0-1,n1-1,n2-1]. */
 int hy3d_mc_cases(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n1, int32_t n2, float level,
                   uint8_t* d_cases);
