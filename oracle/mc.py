@@ -47,11 +47,21 @@ def marching_cubes(vol: np.ndarray, level: float = 0.0, method: str = "lewiner")
         raise ValueError("Input volume should be a 3D numpy array.")
     if level < vol.min() or level > vol.max():
         raise ValueError("Surface level must be within volume data range.")
+    verts, faces = marching_cubes_raw(vol, level)
+    if len(faces) == 0:
+        raise RuntimeError("No surface found at the given iso value.")
+    return verts, faces, None, None
+
+
+def marching_cubes_raw(vol: np.ndarray, level: float = 0.0):
+    """``marching_cubes`` without skimage's argument checks: ``(verts[V,3] float32 in index units, faces[F,3] int32)``,
+    empty arrays when nothing crosses ``level`` — the form ``hy3d_mc_count`` / ``hy3d_mc_emit`` return with a unit
+    transform."""
     lib = _load()
-    pv, pf = ctypes.c_void_p(), ctypes.c_void_p()
-    nv, nf = ctypes.c_int64(), ctypes.c_int64()
-    rc = lib.hy3d_oracle_mc(vol.ctypes.data, vol.shape[0], vol.shape[1], vol.shape[2], float(level),
-                            ctypes.byref(pv), ctypes.byref(nv), ctypes.byref(pf), ctypes.byref(nf))
+    pv, pf, nv, nf = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_int64(), ctypes.c_int64()
+    vol = np.ascontiguousarray(vol, np.float32)
+    rc = lib.hy3d_oracle_mc(vol.ctypes.data, *vol.shape, float(level), ctypes.byref(pv), ctypes.byref(nv), ctypes.byref(pf),
+                            ctypes.byref(nf))
     if rc != 0:
         raise MemoryError("oracle marching cubes")
     V, Fc = nv.value, nf.value
@@ -59,9 +69,7 @@ def marching_cubes(vol: np.ndarray, level: float = 0.0, method: str = "lewiner")
     faces = np.ctypeslib.as_array(ctypes.cast(pf, ctypes.POINTER(ctypes.c_int32)), shape=(max(Fc, 1), 3))[:Fc].copy()
     lib.hy3d_oracle_free(pv)
     lib.hy3d_oracle_free(pf)
-    if Fc == 0:
-        raise RuntimeError("No surface found at the given iso value.")
-    return verts, faces, None, None
+    return verts, faces
 
 
 def cube_cases(vol: np.ndarray, level: float = 0.0) -> np.ndarray:

@@ -17,6 +17,21 @@ from __future__ import annotations
 import numpy as np
 
 
+def bits_equal(a: np.ndarray, b: np.ndarray) -> bool:
+    """Same shape and the same float32 bit patterns (NaN payloads included)."""
+    return a.shape == b.shape and np.array_equal(a.view(np.uint32), b.view(np.uint32))
+
+
+def assert_same_mesh(got, ref):
+    """(verts, faces) pairs: identical faces; vertices NaN at the same places and bit-identical elsewhere (the NaN payload
+    of a vertex interpolated from a NaN sample is not part of the contract)."""
+    (v, f), (vo, fo) = got, ref
+    assert v.shape == vo.shape and np.array_equal(f, fo)
+    nan = np.isnan(v)
+    assert np.array_equal(nan, np.isnan(vo))
+    assert np.array_equal(v[~nan].view(np.uint32), vo[~nan].view(np.uint32))
+
+
 def export_clean(mesh_v: np.ndarray, mesh_f: np.ndarray, flip_winding: bool = True):
     v = np.asarray(mesh_v)
     f = np.asarray(mesh_f)

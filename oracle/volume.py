@@ -263,3 +263,61 @@ def flashvdm_decode(decode_group: Callable, bounds=1.01, num_chunks=10000, mc_le
     grid = grid.copy()
     grid[grid == SENTINEL] = np.nan
     return (grid, stats) if return_stats else grid
+
+
+def flash_layout_reference(index: np.ndarray, n: int, cell: np.ndarray, bmin: np.ndarray, stride: int):
+    """Host restatement of vd:394-412 for the padded layout of ``hy3d_flash_layout_bins``: oracle bin ids, stable sort,
+    128-padding, samples -> (padded index, per-tile group, samples, sample offsets, per-bin counts)."""
+    idx = np.stack(np.unravel_index(index.astype(np.int64), (n, n, n)), 1)
+    pts = (idx.astype(np.float32) * cell.astype(np.float32) + bmin.astype(np.float32)).astype(np.float32)
+    with np.errstate(all="ignore"):
+        bins = flash_bins(pts)
+    bins = np.clip(bins, 0, 215)
+    order = np.argsort(bins, kind="stable")
+    counts = np.bincount(bins, minlength=216)
+    cap = (len(index) + 216 * 127 + 127) // 128 * 128
+    pidx = np.full(cap, -1, np.int32)
+    tile_group = np.full(cap // 128, 215, np.int32)
+    samples, soff, pos, at = [], [0], 0, 0
+    for g in range(216):
+        members = index[order[at:at + counts[g]]]
+        at += counts[g]
+        pc = (counts[g] + 127) // 128 * 128
+        pidx[pos:pos + counts[g]] = members
+        tile_group[pos // 128:(pos + pc) // 128] = g
+        pos += pc
+        samples.append(members[::stride])
+        soff.append(soff[-1] + len(samples[-1]))
+    return pidx, tile_group, np.concatenate(samples).astype(np.int32), np.asarray(soff, np.int32), counts.astype(np.int32)
+
+
+def check_sparse_levels(dec, out, ref=None, tol=None, mc_level=0.0, exact=False, tie_frac=0.0):
+    """A sparse decoder's grid against the reference's.  The active sets are a discontinuous function of the coarse
+    values (sign changes, |v| < 0.95), so with fp16-operand logits (error up to `tol`) a voxel within `tol` of a threshold
+    may flip and carry its fine neighbourhood in or out of the visited set.  What must hold:
+      * exact (fp32 chain): the visited set IS the reference's;
+      * always: every level's visited set is exactly what the reference logic (oracle, bit-pinned to the reference) derives
+        from OUR previous level — "active-cell sets bit-exact given the same field";
+      * every voxel both visited agrees within `tol`; the sets differ on < 1 % of the visited voxels.
+    `dec` ran with ``keep_levels=True``; `ref` None checks the level chain alone (no reference grid at that size).
+    `tie_frac` (FlashVDM only): the fraction of voxels allowed above `tol` (never above 5 x `tol`) — a near-tie of the KV
+    selection (rank 256 vs 257 of the mean similarity, p vs 1e-6) resolves differently under 1e-5 changes of the latents
+    and moves the logits of that one bin; the reference is exactly as sensitive to its own latents."""
+    vis = ~np.isnan(out)
+    lv = [g.cpu().numpy() for g in dec.last_levels]
+    for k in range(len(lv) - 1):
+        want = refine_active_set(lv[k], mc_level, last=(k == len(lv) - 2), nf=lv[k + 1].shape[0])
+        assert np.array_equal(want, lv[k + 1] != SENTINEL), f"level {k + 1}: active set is not the reference logic's for the same field"
+    assert np.array_equal(vis, lv[-1] != SENTINEL)
+    if ref is None:
+        return
+    rvis = ~np.isnan(ref)
+    if exact:
+        assert np.array_equal(vis, rvis), "visited set differs from the reference"
+    both = vis & rvis
+    assert (vis ^ rvis).sum() < 0.01 * rvis.sum(), ((vis ^ rvis).sum(), rvis.sum())
+    err = np.abs(out[both] - ref[both])
+    if tie_frac > 0:
+        assert err.max() < 5 * tol and (err > tol).mean() <= tie_frac, (err.max(), (err > tol).mean())
+    else:
+        assert err.max() < tol, err.max()

@@ -10,6 +10,7 @@ import pytest
 import torch
 
 from oracle import dmc as OD, mc as OM
+from oracle.mesh import assert_same_mesh
 
 ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 
@@ -115,14 +116,6 @@ def gpu_dmc(ctx, vol):
     f = torch.empty((nf, 3), dtype=torch.int32, device="cuda")
     ctx.dmc_emit(v, f)
     return v.cpu().numpy(), f.cpu().numpy()
-
-
-def assert_same_mesh(got, ref):
-    (v, f), (vo, fo) = got, ref
-    assert v.shape == vo.shape and np.array_equal(f, fo)
-    nan = np.isnan(v)
-    assert np.array_equal(nan, np.isnan(vo))
-    assert np.array_equal(v[~nan].view(np.uint32), vo[~nan].view(np.uint32))
 
 
 NOISE_SHAPES = [(5, 6, 97), (4, 5, 300), (3, 4, 600), (2, 7, 40), (9, 2, 33), (3, 3, 3), (2, 2, 70), (6, 3, 2)]

@@ -17,6 +17,7 @@ from hy3dgeo import _lib, weights as W
 from hy3dgeo.surface_extractors import MCSurfaceExtractor
 from hy3dgeo.volume_decoders import HierarchicalVolumeDecoding, VanillaVolumeDecoder, bind
 from oracle import decoder as OD, mc as OM, volume as OV
+from oracle.mesh import bits_equal
 
 pytestmark = pytest.mark.gpu
 CFG = {"mini": W.MINI, "full": W.FULL, "turbo": W.MINI_TURBO}
@@ -48,23 +49,6 @@ def gpu_mc(ctx, vol, level, div=(1, 1, 1), mul=(1, 1, 1), add=(0, 0, 0)):
     return v.cpu().numpy(), f.cpu().numpy(), mm
 
 
-def oracle_mc_raw(vol, level):
-    import ctypes
-    lib = OM._load()
-    pv, pf, nv, nf = ctypes.c_void_p(), ctypes.c_void_p(), ctypes.c_int64(), ctypes.c_int64()
-    vol = np.ascontiguousarray(vol, np.float32)
-    lib.hy3d_oracle_mc(vol.ctypes.data, *vol.shape, float(level), ctypes.byref(pv), ctypes.byref(nv), ctypes.byref(pf), ctypes.byref(nf))
-    V, Fc = nv.value, nf.value
-    verts = np.ctypeslib.as_array(ctypes.cast(pv, ctypes.POINTER(ctypes.c_float)), shape=(max(V, 1), 3))[:V].copy()
-    faces = np.ctypeslib.as_array(ctypes.cast(pf, ctypes.POINTER(ctypes.c_int32)), shape=(max(Fc, 1), 3))[:Fc].copy()
-    lib.hy3d_oracle_free(pv); lib.hy3d_oracle_free(pf)
-    return verts, faces
-
-
-def bits_equal(a, b):
-    return a.shape == b.shape and np.array_equal(a.view(np.uint32), b.view(np.uint32))
-
-
 # ------------------------------------------------------------------------------ marching cubes
 @pytest.mark.parametrize("shape,level", [((2, 2, 2), 0.0), ((3, 5, 33), 0.1), ((17, 9, 32), 0.0), ((9, 31, 65), -0.2),
                                          ((20, 21, 97), 0.0), ((6, 7, 300), 0.05), ((4, 5, 600), 0.0)])
@@ -75,7 +59,7 @@ def test_mc_random_fields_bit_exact(ctx, shape, level):
     vol = rng.standard_normal(shape).astype(np.float32)
     assert np.array_equal(ctx.mc_cases(torch.from_numpy(vol).cuda(), level).cpu().numpy(), OM.cube_cases(vol, level))
     v, f, _ = gpu_mc(ctx, vol, level)
-    vo, fo = oracle_mc_raw(vol, level)
+    vo, fo = OM.marching_cubes_raw(vol, level)
     assert bits_equal(v, vo) and np.array_equal(f, fo)
 
 
@@ -83,13 +67,13 @@ def test_mc_sphere_nan_and_exact_zero(ctx):
     vol = sphere(65)
     vol[10, 10, 10] = 0.0                                   # exact level value: "v - level > 0" is false
     v, f, mm = gpu_mc(ctx, vol, 0.0)
-    vo, fo = oracle_mc_raw(vol, 0.0)
+    vo, fo = OM.marching_cubes_raw(vol, 0.0)
     assert bits_equal(v, vo) and np.array_equal(f, fo) and f.shape[0] == 2 * v.shape[0] - 4
     assert mm[0] == vol.min() and mm[1] == vol.max() and mm[2] is False
     nanv = vol.copy()
     nanv[np.abs(nanv) > 0.999] = np.nan                     # unvisited voxels of the sparse decoders
     v, f, mm = gpu_mc(ctx, nanv, 0.0)
-    vo, fo = oracle_mc_raw(nanv, 0.0)
+    vo, fo = OM.marching_cubes_raw(nanv, 0.0)
     assert bits_equal(v, vo) and np.array_equal(f, fo) and mm[2] is True and np.isnan(v).any()
 
 
@@ -417,31 +401,6 @@ def test_flashvdm_level0_selection_and_logits(dev, ctx):
         assert d < (LOGIT_TOL if g not in bad_groups else 2e-2), (g, d)
 
 
-def _layout_reference(index, n, cell, bmin, stride):
-    """Host restatement of reference vd:394-412 for the padded layout: oracle bin ids, stable sort, 128-padding, samples."""
-    idx = np.stack(np.unravel_index(index.astype(np.int64), (n, n, n)), 1)
-    pts = (idx.astype(np.float32) * cell.astype(np.float32) + bmin.astype(np.float32)).astype(np.float32)
-    with np.errstate(all="ignore"):
-        bins = OV.flash_bins(pts)
-    bins = np.clip(bins, 0, 215)
-    order = np.argsort(bins, kind="stable")
-    counts = np.bincount(bins, minlength=216)
-    cap = (len(index) + 216 * 127 + 127) // 128 * 128
-    pidx = np.full(cap, -1, np.int32)
-    tile_group = np.full(cap // 128, 215, np.int32)
-    samples, soff, pos, at = [], [0], 0, 0
-    for g in range(216):
-        members = index[order[at:at + counts[g]]]
-        at += counts[g]
-        pc = (counts[g] + 127) // 128 * 128
-        pidx[pos:pos + counts[g]] = members
-        tile_group[pos // 128:(pos + pc) // 128] = g
-        pos += pc
-        samples.append(members[::stride])
-        soff.append(soff[-1] + len(samples[-1]))
-    return pidx, tile_group, np.concatenate(samples).astype(np.int32), np.asarray(soff, np.int32), counts.astype(np.int32)
-
-
 @pytest.mark.parametrize("case", ["shell", "random", "flat_axis", "tiny", "empty"])
 def test_flash_layout_bins_matches_reference_restatement(case, dev, ctx):
     """hy3d_flash_layout_bins: bin ids, stable order, padding, per-tile group and stride samples, bit for bit."""
@@ -464,7 +423,7 @@ def test_flash_layout_bins_matches_reference_restatement(case, dev, ctx):
     for stride in (50, 30):
         pidx, tg, sidx, soff, counts = ctx.flash_layout_bins(torch.from_numpy(index).to(dev), (n, n, n), cell, bmin, stride, with_counts=True)
         if len(index):
-            rp, rt, rs, ro, rc = _layout_reference(index, n, cell, bmin, stride)
+            rp, rt, rs, ro, rc = OV.flash_layout_reference(index, n, cell, bmin, stride)
         else:
             rp, rt = np.full(pidx.numel(), -1, np.int32), np.full(tg.numel(), 215, np.int32)
             rs, ro, rc = np.zeros(0, np.int32), np.zeros(217, np.int32), np.zeros(216, np.int32)
@@ -539,34 +498,6 @@ def test_refine_odd_levels_matches_oracle(ctx):
         ctx.refine_level(torch.from_numpy(base).cuda(), 0.0, True, None, 2 * 18 + 1)
 
 
-def check_sparse_levels(dec, out, ref, tol, mc_level=0.0, exact=False, tie_frac=0.0):
-    """A sparse decoder's grid against the reference's.  The active sets are a discontinuous function of the coarse
-    values (sign changes, |v| < 0.95), so with fp16-operand logits (error up to `tol`) a voxel within `tol` of a threshold
-    may flip and carry its fine neighbourhood in or out of the visited set.  What must hold:
-      * exact (fp32 chain): the visited set IS the reference's;
-      * always: every level's visited set is exactly what the reference logic (oracle, bit-pinned to the reference) derives
-        from OUR previous level — "active-cell sets bit-exact given the same field";
-      * every voxel both visited agrees within `tol`; the sets differ on < 1 % of the visited voxels.
-    `tie_frac` (FlashVDM only): the fraction of voxels allowed above `tol` (never above 5 x `tol`) — a near-tie of the KV
-    selection (rank 256 vs 257 of the mean similarity, p vs 1e-6) resolves differently under 1e-5 changes of the latents
-    and moves the logits of that one bin; the reference is exactly as sensitive to its own latents."""
-    vis, rvis = ~np.isnan(out), ~np.isnan(ref)
-    lv = [g.cpu().numpy() for g in dec.last_levels]
-    for k in range(len(lv) - 1):
-        want = OV.refine_active_set(lv[k], mc_level, last=(k == len(lv) - 2), nf=lv[k + 1].shape[0])
-        assert np.array_equal(want, lv[k + 1] != OV.SENTINEL), f"level {k + 1}: active set is not the reference logic's for the same field"
-    assert np.array_equal(vis, lv[-1] != OV.SENTINEL)
-    if exact:
-        assert np.array_equal(vis, rvis), "visited set differs from the reference"
-    both = vis & rvis
-    assert (vis ^ rvis).sum() < 0.01 * rvis.sum(), ((vis ^ rvis).sum(), rvis.sum())
-    err = np.abs(out[both] - ref[both])
-    if tie_frac > 0:
-        assert err.max() < 5 * tol and (err > tol).mean() <= tie_frac, (err.max(), (err > tol).mean())
-    else:
-        assert err.max() < tol, err.max()
-
-
 def _sparse_vae(tag, g, dev):
     cfg = CFG[tag]
     sd = W.sparsify_field(W.synthetic_state_dict(cfg, seed=0), cfg, int(g["keep_freqs"]), float(g["gain"]), float(g["bias"]))
@@ -593,7 +524,7 @@ def test_hierarchical_three_levels_matches_patched_reference(res, minres, gold, 
                   enable_pbar=False)[0].cpu().numpy()
         ctx.check_watchdog()
         assert out.shape == ref.shape and len(dec.last_stats[0]["levels"]) == 3
-        check_sparse_levels(dec, out, ref, tol, exact=exact)
+        OV.check_sparse_levels(dec, out, ref, tol, exact=exact)
         if exact:
             assert dec.last_stats[0]["queries"] == list(g[f"hier{res}_queries"])
     ctx.set_precision(_lib.PRECISION_FP16_TC)
