@@ -111,6 +111,10 @@ SYMBOLS = {
     "hy3d_dmc_count": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32,
                                  C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_float)]),
     "hy3d_dmc_emit": (C.c_int, [C.c_void_p, c_f32p, c_i32p]),
+    "hy3d_dmc_count_slab": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32, C.c_int32,
+                                      C.POINTER(C.c_int64), C.POINTER(C.c_int64), C.POINTER(C.c_float)]),
+    "hy3d_dmc_emit_slab": (C.c_int, [C.c_void_p, C.c_int64, c_f32p, c_i32p, c_i32p]),
+    "hy3d_dmc_center": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, C.POINTER(C.c_int32)]),
     "hy3d_mesh_clean": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int32, c_f32p, c_i32p,
                                   C.POINTER(C.c_int64), C.POINTER(C.c_int64)]),
     "hy3d_mesh_remove_floaters": (C.c_int, [C.c_void_p, c_f32p, C.c_int64, c_i32p, C.c_int64, C.c_int64, c_f32p, c_i32p,
@@ -604,6 +608,28 @@ class GeoContext:
     def dmc_emit(self, verts: torch.Tensor, faces: torch.Tensor):
         self.sync_stream()
         self._check(self.lib.hy3d_dmc_emit(self.h, _ptr(verts), _ptr(faces)), "hy3d_dmc_emit")
+
+    def dmc_count_slab(self, slab: torch.Tensor, own_planes: int, plane0: int, n0_global: int):
+        """slab = owned planes [plane0, plane0 + own_planes) of a grid of n0_global planes, followed by the next slab's
+        halo planes; -> (nV, nF, (min, max, nan)) of the owned part (see hy3dgeo.h: hy3d_dmc_count_slab)."""
+        self.sync_stream()
+        nv, nf = C.c_int64(), C.c_int64()
+        mm = (C.c_float * 3)()
+        self._check(self.lib.hy3d_dmc_count_slab(self.h, _ptr(slab), int(own_planes), slab.shape[0] - int(own_planes), slab.shape[1],
+                                                 slab.shape[2], int(plane0), int(n0_global), C.byref(nv), C.byref(nf), mm),
+                    "hy3d_dmc_count_slab")
+        return nv.value, nf.value, (mm[0], mm[1], bool(mm[2]))
+
+    def dmc_emit_slab(self, id_base: int, verts: torch.Tensor, faces: torch.Tensor, bbox: torch.Tensor):
+        """Uncentred vertices, faces with global ids, and the slab's ordered-int bounding box (int32 [6], device)."""
+        self.sync_stream()
+        self._check(self.lib.hy3d_dmc_emit_slab(self.h, int(id_base), _ptr(verts), _ptr(faces), _ptr(bbox)), "hy3d_dmc_emit_slab")
+
+    def dmc_center(self, verts: torch.Tensor, bbox6):
+        """verts -= 0.5f * (lo + hi) in place; bbox6 = 6 ordered ints (lo[3], hi[3]) on the host."""
+        self.sync_stream()
+        box = (C.c_int32 * 6)(*[int(v) for v in bbox6])
+        self._check(self.lib.hy3d_dmc_center(self.h, _ptr(verts), verts.shape[0], box), "hy3d_dmc_center")
 
     def mesh_clean(self, verts: torch.Tensor, faces: torch.Tensor, flip_winding: bool):
         """Device tensors (verts float32 [V,3], faces int32 [F,3]) -> the same mesh without non-finite / unreferenced

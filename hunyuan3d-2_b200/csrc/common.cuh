@@ -105,11 +105,13 @@ struct McState {
   DevBuf bits, rowcnt, rowoff, stats;
 };
 
-struct DmcState {                     // dual marching cubes (dmc.cu): hy3d_dmc_count -> hy3d_dmc_emit
+struct DmcState {                     // dual marching cubes (dmc.cu): hy3d_dmc_count[_slab] -> hy3d_dmc_emit[_slab]
   bool counted = false;
   const float* grid = nullptr;
-  int n0 = 0, n1 = 0, n2 = 0, words = 0;
-  long long nV = 0, nF = 0;
+  int n0 = 0, n1 = 0, n2 = 0, words = 0;   // n0: local planes (owned + read halo)
+  int plane0 = 0, N0 = 0, own = 0;    // slab: global index of local plane 0, global plane count, owned planes
+  long long nV = 0, nF = 0;           // owned vertices, faces
+  long long nVall = 0;                // vertices of every local cube plane (the owned ones and the halo's first)
   DevBuf bits, rowcnt, rowoff, stats, rec;
 };
 

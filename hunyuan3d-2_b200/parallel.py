@@ -172,9 +172,11 @@ def extract_mesh_sharded(local: torch.Tensor, plane0: int, count_slab: Callable,
     count_slab : (slab_with_halo, own_planes) -> (nV, nF, (vmin, vmax, has_nan))     (MCSurfaceExtractor.count_slab)
     emit_slab  : (nV, nF, plane0, id_base) -> (verts [nV, 3] float32, faces [nF, 3] int32), face ids global
     Returns (verts, faces) on ``dst`` (a group rank) — exactly the mesh of the whole grid: rank pieces are contiguous
-    ranges of the global lexicographic vertex / face order — and None elsewhere.  Raises the errors of
-    ``skimage.measure.marching_cubes`` (level outside the data range, no surface) on every rank alike; a rank whose
-    own kernels fail makes ALL ranks raise before the mesh exchange (nobody is left blocked in a collective)."""
+    ranges of the global lexicographic vertex / face order — and None elsewhere; with ``dst=None`` every rank receives
+    the mesh (one all-gather of the vertex pieces and one of the face pieces).  Raises the errors of
+    ``skimage.measure.marching_cubes`` (level outside the data range, no surface) on every rank alike; ``mc_level=None``
+    skips the range check (dual marching cubes has no level).  A rank whose own kernels fail makes ALL ranks raise before
+    the mesh exchange (nobody is left blocked in a collective)."""
     rank, world = dist.get_rank(group), dist.get_world_size(group)
     own = local.shape[0] - (MC_HALO if with_halo and rank < world - 1 else 0)
     slab = local if with_halo else exchange_halo(local, MC_HALO, group)
@@ -195,9 +197,9 @@ def extract_mesh_sharded(local: torch.Tensor, plane0: int, count_slab: Callable,
         raise RuntimeError("marching cubes failed on another rank of the group")
     nvs, nfs = [int(v) for v in allst[:, 0]], [int(v) for v in allst[:, 1]]
     gmin, gmax, any_nan = float(allst[:, 2].min()), float(allst[:, 3].max()), bool(allst[:, 4].max() > 0)
-    if not any_nan and (mc_level < gmin or mc_level > gmax):
+    if mc_level is not None and not any_nan and (mc_level < gmin or mc_level > gmax):
         raise ValueError("Surface level must be within volume data range.")
-    if sum(nfs) == 0:
+    if sum(nfs) == 0 and sum(nvs) == 0:        # marching cubes has faces iff it has vertices; a DMC mesh may have no face
         raise RuntimeError("No surface found at the given iso value.")
     verts = faces = None
     try:
@@ -206,6 +208,10 @@ def extract_mesh_sharded(local: torch.Tensor, plane0: int, count_slab: Callable,
         err = e
     if not agree(err is None, local.device, group):
         raise err if err is not None else RuntimeError("marching cubes failed on another rank of the group")
+    if dst is None:
+        V = all_gather_ranges(verts.reshape(-1), [3 * v for v in nvs], group).view(-1, 3)
+        F = all_gather_ranges(faces.reshape(-1), [3 * f for f in nfs], group).view(-1, 3) if sum(nfs) else faces
+        return V, F
     # mesh pieces -> dst: one batched group of point-to-point copies (sizes differ per rank)
     sends, recvs, V, F = [], [], None, None
     if rank == dst:
@@ -245,7 +251,7 @@ def decode_list_sharded(decode_values: Callable[[torch.Tensor], torch.Tensor], i
 class SlabGrid:
     """A batch of occupancy grids left partitioned along axis 0 across a process group — the opaque grid of SURVEY §8b:
     it answers ``shape`` / ``len`` / ``[i]`` like the ``[B, N, N, N]`` tensor the reference decoders return, the B200
-    ``MCSurfaceExtractor`` recognises it and extracts the mesh slab by slab (``extract_mesh_sharded``), and
+    ``MCSurfaceExtractor`` and ``DMCSurfaceExtractor`` recognise it and extract the mesh slab by slab (``extract_mesh_sharded``), and
     ``to_tensor()`` materialises the ordinary tensor on every rank for any other consumer.
 
     slabs[b]  : this rank's planes [plane0, plane0 + own) of item b, followed by the next slab's first MC_HALO planes

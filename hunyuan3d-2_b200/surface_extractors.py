@@ -157,12 +157,13 @@ class DMCSurfaceExtractor(SurfaceExtractor):
     oriented like ``MCSurfaceExtractor``'s mesh so that ``export_to_trimesh``'s flip serves both; vertices centred on
     their bounding box.  ``mc_level`` and ``bounds`` play no part, as in the reference.  NaN voxels count as outside;
     vertices on their rim come out NaN, as with ``mc``.  The contract is ``oracle/dmc.py``; diso's own triangles, vertex
-    order and quad split are not reproduced (DESIGN.md §2).  A ``SlabGrid`` is gathered to one tensor first."""
+    order and quad split are not reproduced (DESIGN.md §2).  A ``SlabGrid`` is extracted slab by slab (``run_sharded``)
+    and every rank receives the whole mesh."""
 
     def run_device(self, grid_logit, **kwargs):
         """Returns device tensors (verts float32 [V,3], faces int32 [F,3])."""
         if type(grid_logit).__name__ == "SlabGrid":
-            grid_logit = grid_logit.to_tensor()[0]
+            return self.run_sharded(grid_logit)
         if not isinstance(grid_logit, torch.Tensor) or not grid_logit.is_cuda:
             raise RuntimeError("DMCSurfaceExtractor needs a CUDA tensor (hy3dgeo has no CPU path)")
         if grid_logit.dim() != 3:
@@ -179,6 +180,44 @@ class DMCSurfaceExtractor(SurfaceExtractor):
 
     def run(self, grid_logit, **kwargs):
         return _to_host(*self.run_device(grid_logit, **kwargs))
+
+    def run_sharded(self, grid):
+        """``grid``: a one-item ``hy3dgeo.parallel.SlabGrid``.  Every rank extracts the vertices of the cubes based at its
+        planes and the faces of its edge planes (``hy3d_dmc_count_slab`` / ``hy3d_dmc_emit_slab``, behind the two-plane
+        halo of ``extract_mesh_sharded``), the slabs' bounding boxes are reduced, and every rank receives the pieces and
+        centres the whole mesh: device tensors equal bit for bit to ``run_device`` on the gathered tensor.  Errors are raised
+        on every rank alike."""
+        import torch.distributed as dist
+        from .parallel import _staged, extract_mesh_sharded
+        slab = grid.slabs[0]
+        if slab.dim() != 3:
+            raise ValueError("Input volume should be a 3D array.")
+        if not slab.is_cuda:
+            raise RuntimeError("DMCSurfaceExtractor needs a CUDA tensor (hy3dgeo has no CPU path)")
+        dev, n0 = slab.device, grid.dims[0]
+        ctx = get_context(dev)
+        bbox = torch.empty(6, dtype=torch.int32, device=dev)
+        keep = []
+
+        def count_slab(s, own):
+            keep.append(s.detach().to(torch.float32).contiguous())         # read again by the emit
+            return ctx.dmc_count_slab(keep[-1], own, grid.plane0, n0)
+
+        def emit_slab(nv, nf, plane0, id_base):
+            verts = torch.empty((nv, 3), dtype=torch.float32, device=dev)
+            faces = torch.empty((nf, 3), dtype=torch.int32, device=dev)
+            ctx.dmc_emit_slab(id_base, verts, faces, bbox)
+            return verts, faces
+
+        verts, faces = extract_mesh_sharded(slab, grid.plane0, count_slab, emit_slab, None, grid.group, dst=None,
+                                            with_halo=grid.with_halo)
+        # box of the whole mesh: min of lo, max of hi (as min of -hi) over the slabs, in ordered ints
+        box = torch.cat([bbox[:3].to(torch.int64), -bbox[3:].to(torch.int64)])
+        box = box.cpu() if _staged(box, grid.group) else box
+        dist.all_reduce(box, op=dist.ReduceOp.MIN, group=grid.group)
+        lo_hi = box.cpu().tolist()
+        ctx.dmc_center(verts, lo_hi[:3] + [-v for v in lo_hi[3:]])
+        return verts, faces
 
 
 def export_to_trimesh(mesh_output, device=None):

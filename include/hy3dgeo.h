@@ -266,6 +266,26 @@ int hy3d_dmc_count(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n1, i
  * lexicographic (edge owner voxel, edge axis) order, oriented like hy3d_mc_emit's.  d_verts: fp32 [V,3]; d_faces:
  * int32 [F,3]. */
 int hy3d_dmc_emit(hy3d_ctx* ctx, float* d_verts, int32_t* d_faces);
+/* Slab forms for grids partitioned along axis 0 across GPUs (no reference counterpart: the reference is single-device).
+ * d_slab holds planes [plane0, plane0 + own_planes + halo_planes) of a grid of n0_global planes: the first own_planes are
+ * OWNED by this slab, the rest are the next slab's first planes, kept as a halo; halo_planes must be at least
+ * min(2, n0_global - plane0 - own_planes) (planes past the second are not read).  A slab owns
+ *   the vertices of the cubes based at its planes [plane0, plane0 + own_planes), and
+ *   the faces of the edges in planes [plane0 + 1, plane0 + own_planes + 1) (from plane 0 on the first slab),
+ * so the vertices and faces of consecutive slabs concatenate into exactly the mesh of hy3d_dmc_count / hy3d_dmc_emit when
+ * each slab passes  id_base = number of vertices owned by all earlier slabs  (faces of the last edge plane reference
+ * vertices of the first halo cube plane, whose ids continue past this slab's own count).  Coordinates and interior tests
+ * use global plane indices.  hy3d_dmc_count_slab returns the owned counts, as hy3d_dmc_count does; bad plane ranges
+ * return HY3D_ERR_ARG.
+ * hy3d_dmc_emit_slab writes the vertices NOT centred, and the bounding box of its non-NaN vertices to d_bbox_out (device
+ * int32[6]: lo[3], hi[3] as ordered ints, i.e. the float bits with negative values XORed by 0x7fffffff so that integer
+ * order is float order; an empty box is {INT32_MAX x3, INT32_MIN x3}).  The box of the whole mesh is the min of the
+ * slabs' lo and the max of their hi; hy3d_dmc_center(ctx, d_verts, n_verts, h_bbox6) then subtracts 0.5f * (lo + hi) from
+ * n_verts vertices in fp32 (h_bbox6 in HOST memory, same encoding), which is what hy3d_dmc_emit does with the grid's box. */
+int hy3d_dmc_count_slab(hy3d_ctx* ctx, const float* d_slab, int32_t own_planes, int32_t halo_planes, int32_t n1, int32_t n2,
+                        int32_t plane0, int32_t n0_global, int64_t* h_num_verts, int64_t* h_num_faces, float h_minmax[3]);
+int hy3d_dmc_emit_slab(hy3d_ctx* ctx, int64_t id_base, float* d_verts, int32_t* d_faces, int32_t* d_bbox_out);
+int hy3d_dmc_center(hy3d_ctx* ctx, float* d_verts, int64_t n_verts, const int32_t h_bbox6[6]);
 /* ---- mesh clean-up: the device side of export_to_trimesh (hy3dgen/shapegen/pipelines.py:95-110) ---------------------
  * `mesh_f[:, ::-1]` (flip_winding != 0) and what trimesh.Trimesh(v, f)'s default processing does to a mesh with
  * non-finite vertices: faces that reference a NaN / inf vertex are dropped, then vertices that are non-finite or no longer
