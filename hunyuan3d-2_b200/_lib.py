@@ -126,11 +126,8 @@ SYMBOLS = {
     "hy3d_profile": (C.c_int, [C.c_void_p, C.c_int]),
     "hy3d_profile_read": (C.c_int, [C.c_void_p, C.POINTER(C.c_double), C.POINTER(C.c_int64)]),
     "hy3d_debug_watchdog": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
-    "hy3d_debug_retain": (C.c_int, [C.c_void_p, C.c_int]),
-    "hy3d_debug_experiment": (C.c_int, [C.c_void_p, C.c_int, C.c_int]),
-    "hy3d_debug_timers": (C.c_int, [C.c_void_p, C.POINTER(C.c_uint64)]),
+    "hy3d_debug_force_online_softmax": (C.c_int, [C.c_void_p, C.c_int]),
     "hy3d_debug_attn_redo": (C.c_int, [C.c_void_p, C.POINTER(C.c_int32)]),
-    "hy3d_debug_fetch": (C.c_int, [C.c_void_p, C.c_int, c_f32p, C.c_int64, C.POINTER(C.c_int32)]),
     "hy3d_mc_cases": (C.c_int, [C.c_void_p, c_f32p, C.c_int32, C.c_int32, C.c_int32, C.c_float, C.c_void_p]),
 }
 
@@ -403,28 +400,14 @@ class GeoContext:
         self._check(self.lib.hy3d_profile_read(self.h, ms, cnt), "hy3d_profile_read")
         return {f: (ms[i], cnt[i]) for i, f in enumerate(self.FAMILIES)}
 
-    def debug_experiment(self, bits: int = 0, attn_poly: int = 0):
-        self._check(self.lib.hy3d_debug_experiment(self.h, int(bits), int(attn_poly)), "hy3d_debug_experiment")
-
-    def debug_timers(self):
-        out = (C.c_uint64 * 32)()
-        self._check(self.lib.hy3d_debug_timers(self.h, out), "hy3d_debug_timers")
-        return list(out)
+    def debug_force_online_softmax(self, enable: bool):
+        """Run every attention launch of this context on the online-softmax kernel (tests use it as a reference)."""
+        self._check(self.lib.hy3d_debug_force_online_softmax(self.h, int(enable)), "hy3d_debug_force_online_softmax")
 
     def debug_attn_redo(self) -> int:
         n = C.c_int32()
         self._check(self.lib.hy3d_debug_attn_redo(self.h, C.byref(n)), "hy3d_debug_attn_redo")
         return int(n.value)
-
-    def debug_retain(self, enable: bool):
-        self._check(self.lib.hy3d_debug_retain(self.h, int(enable)), "hy3d_debug_retain")
-
-    def debug_fetch(self, stage: int, rows: int, max_width: int = 8192) -> torch.Tensor:
-        self.sync_stream()
-        out = torch.empty(rows * max_width, dtype=torch.float32, device=self.device)
-        w = C.c_int32()
-        self._check(self.lib.hy3d_debug_fetch(self.h, stage, _ptr(out), rows, C.byref(w)), "hy3d_debug_fetch")
-        return out[: rows * w.value].view(rows, w.value)
 
     def check_watchdog(self):
         rec = self.watchdog()

@@ -1,6 +1,5 @@
 // C-ABI glue of libhy3dgeo.so: context, weights, decoder entry points (include/hy3dgeo.h).
 #include <cstdarg>
-#include <cstdlib>
 
 #include "common.cuh"
 
@@ -12,32 +11,6 @@ int hy3d_fail(hy3d_ctx* ctx, int code, const char* fmt, ...) {
   va_end(ap);
   if (ctx) ctx->err = buf;
   return code;
-}
-
-int hy3d_debug_keep(hy3d_ctx* ctx, int stage, const void* src, size_t bytes, int layout, long long rows, int width) {
-  if (!ctx->debug_retain) return 0;
-  HY3D_CUDA(ctx, ctx->dbg[stage].reserve(bytes));
-  HY3D_CUDA(ctx, cudaMemcpyAsync(ctx->dbg[stage].p, src, bytes, cudaMemcpyDeviceToDevice, ctx->stream));
-  ctx->dbg_layout[stage] = layout; ctx->dbg_rows = rows; ctx->dbg_width[stage] = width;
-  return 0;
-}
-
-// R32 [rows/128][W/4][128][4] or T16 (SW128 tiles) -> row-major fp32 [rows, W]
-__global__ void k_debug_unpack(const void* __restrict__ src, int layout, long long rows, int W, float* __restrict__ out) {
-  long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;
-  if (t >= rows * W) return;
-  long long row = t / W; int c = (int)(t % W);
-  long long mb = row / 128; int r = (int)(row % 128);
-  float v;
-  if (layout == 1) {
-    v = reinterpret_cast<const float*>(src)[((mb * (W / 4) + c / 4) * 128 + r) * 4 + (c & 3)];
-  } else {
-    const unsigned char* tile = reinterpret_cast<const unsigned char*>(src) + (mb * (W / 64) + c / 64) * 16384;
-    int cc = c % 64;
-    size_t off = (size_t)(r >> 3) * 1024 + (r & 7) * 128 + (((cc >> 3) ^ (r & 7)) << 4) + (cc & 7) * 2;
-    v = __half2float(*reinterpret_cast<const __half*>(tile + off));
-  }
-  out[t] = v;
 }
 
 extern "C" {
@@ -63,33 +36,9 @@ int hy3d_profile_read(hy3d_ctx* ctx, double h_ms[16], int64_t h_count[16]) {
   return HY3D_OK;
 }
 
-int hy3d_debug_retain(hy3d_ctx* ctx, int enable) {
+int hy3d_debug_force_online_softmax(hy3d_ctx* ctx, int enable) {
   if (!ctx) return HY3D_ERR_ARG;
-  ctx->debug_retain = enable ? 1 : 0;
-  return HY3D_OK;
-}
-
-int hy3d_debug_experiment(hy3d_ctx* ctx, int bits, int attn_poly) {
-  if (!ctx) return HY3D_ERR_ARG;
-  ctx->xbits = bits;
-  ctx->attn_poly = attn_poly;
-  return HY3D_OK;
-}
-
-int hy3d_debug_fetch(hy3d_ctx* ctx, int stage, float* d_out, int64_t rows, int32_t* h_width) {
-  if (!ctx || stage < 0 || stage >= 8 || !d_out || !h_width) return HY3D_ERR_ARG;
-  if (!ctx->dbg[stage].p) return hy3d_fail(ctx, HY3D_ERR_STATE, "stage %d was not retained", stage);
-  HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
-  const int W = ctx->dbg_width[stage];
-  *h_width = W;
-  if (rows > ctx->dbg_rows) return hy3d_fail(ctx, HY3D_ERR_ARG, "only %lld rows retained", ctx->dbg_rows);
-  if (ctx->dbg_layout[stage] == 0) {
-    HY3D_CUDA(ctx, cudaMemcpyAsync(d_out, ctx->dbg[stage].p, (size_t)rows * W * 4, cudaMemcpyDeviceToDevice, ctx->stream));
-  } else {
-    long long total = rows * W;
-    k_debug_unpack<<<(unsigned)ceil_div64(total, 256), 256, 0, ctx->stream>>>(ctx->dbg[stage].p, ctx->dbg_layout[stage], rows, W, d_out);
-    HY3D_LAUNCH_CHECK(ctx);
-  }
+  ctx->force_online_softmax = enable ? 1 : 0;
   return HY3D_OK;
 }
 
@@ -132,9 +81,6 @@ int hy3d_create(int device, void* cuda_stream, hy3d_ctx** out) {
   ctx->device = device;
   ctx->stream = (cudaStream_t)cuda_stream;
   ctx->num_sms = prop.multiProcessorCount;
-  if (const char* e = getenv("HY3D_ATTN_POLY")) ctx->attn_poly = atoi(e);
-  if (const char* e = getenv("HY3D_DBG")) ctx->xbits = atoi(e);
-  if (const char* e = getenv("HY3D_CHUNK")) { long long c = atoll(e); if (c >= 256) ctx->chunk_points = c / 256 * 256; }
   if (cudaMallocHost(&ctx->pinned, 4096) != cudaSuccess) { delete ctx; return HY3D_ERR_CUDA; }
   *out = ctx;
   return HY3D_OK;
@@ -154,7 +100,6 @@ void hy3d_destroy(hy3d_ctx* ctx) {
   ctx->w.fold.release();
   { KVSelState& k = ctx->kvsel; k.ktile.release(); k.vtile.release(); k.ntok.release(); k.sel.release(); k.qs.release(); k.qbar.release(); k.mask.release(); }
   ctx->scratch.release(); ctx->scratch2.release(); ctx->ln_mr.release();
-  for (auto& b : ctx->dbg) b.release();
   for (auto& r : ctx->prof.recs) { cudaEventDestroy(r.e0); cudaEventDestroy(r.e1); }
   for (auto e : ctx->prof.pool) cudaEventDestroy(e);
   if (ctx->pinned) cudaFreeHost(ctx->pinned);
@@ -182,7 +127,7 @@ int64_t hy3d_launch_count(const hy3d_ctx* ctx) { return ctx ? ctx->launches : 0;
 int hy3d_attention_info(hy3d_ctx* ctx, float* h_score_bound, int32_t* h_bounded_kernel, float* h_measured_bound) {
   if (!ctx || !h_score_bound || !h_bounded_kernel) return HY3D_ERR_ARG;
   *h_score_bound = ctx->w.attn_bound;
-  const bool fast = ctx->w.attn_fast && !(ctx->xbits & 0x20);
+  const bool fast = ctx->w.attn_fast && !ctx->force_online_softmax;
   *h_bounded_kernel = !fast ? 0 : (ctx->kv.shifted ? 2 : 1);
   if (h_measured_bound) {
     *h_measured_bound = ctx->w.attn_bound;
@@ -274,7 +219,7 @@ int hy3d_prepare_kv(hy3d_ctx* ctx, const float* d_latents, int32_t M) {
   HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
   // tensor path: K/V projected by the split-precision tcgen05 GEMMs; HY3D_PRECISION_FP32_SIMT (the on-device
   // fp32 statement used as a cross-check) and shapes the tensor path does not tile keep the CUDA-core projection
-  if (ctx->precision != HY3D_PRECISION_FP32_SIMT && ctx->w.t_qp && ctx->w.t_ckv3 && !(ctx->xbits & 0x10000))
+  if (ctx->precision != HY3D_PRECISION_FP32_SIMT && ctx->w.t_qp && ctx->w.t_ckv3)
     return hy3d_tc_project_kv(ctx, d_latents, M);
   if (int rc = hy3d_simt_prepare_kv(ctx, d_latents, M)) return rc;
   return hy3d_tc_prepare_kv(ctx);

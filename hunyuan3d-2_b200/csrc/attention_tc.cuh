@@ -32,7 +32,7 @@
 //    whose best score is >= -5 — every row of a trained or random model — lose < 2^-20 per term).  Two threads per
 //    query row (16 softmax warps) halve the serial latency of each stream; per pair of elements the instruction
 //    stream is 2 MUFU.EX2 + FADD2 + F2FP, or the packed polynomial (3 FADD2 + 3 FFMA2 + 2 IMAD + FADD2 + F2FP) for
-//    kPoly of every 8 pairs.  Heads whose measured bound exceeds 15.9 subtract a per-head shift first (head_shift) and
+//    ATT_POLY_PAIRS of every 8 pairs.  Heads whose measured bound exceeds 15.9 subtract a per-head shift first (head_shift) and
 //    rows that end up far below it are flagged for an exact redo by k_attn_tc (redo_list).
 //  * k_attn_tc — online softmax with a running maximum (lazy rescale) for everything else (no q/k norm, norm gains
 //    beyond the shift range, the redo pass).  Same two-threads-per-row layout; the halves of a row exchange their
@@ -44,6 +44,7 @@ constexpr int TM_S0 = 0, TM_P0 = 256, TM_O0 = 384;
 constexpr int ATT_THREADS = 640;           // k_attn_tc: 4 role warps + 2 x 8 softmax warps (two threads per row)
 constexpr int ATT_FAST_THREADS = 640;      // k_attn_fast: 4 role warps + 2 x 8 softmax warps
 constexpr float ATT_FAST_BOUND = 15.9f;    // exp2(15.9) = 61147 < 65504: no fp16 overflow, ever
+constexpr int ATT_POLY_PAIRS = 2;          // k_attn_fast: pairs of every 8 whose exp2 runs on the FMA pipe (2 and 3 tie, 4 is 3 % slower, 0 11 %)
 
 struct AttnTC {
   const uint8_t* Q;      // T16 [Pb][H]  (q already scaled by 1/sqrt(d) * log2e)
@@ -59,14 +60,12 @@ struct AttnTC {
   // K / V gathered from several GPUs (sequence-parallel latent transformer): tile j of head h lives in chunk j / kv_tpr at
   // K + (j / kv_tpr) * kv_chunk_stride + (h * kv_tpr + j % kv_tpr) * 16 KB (same for V).  kv_tpr = 0: one chunk of nkv tiles.
   int kv_tpr; long long kv_chunk_stride;
-  int no_pipe;           // experiment: load both 32-column halves of S before any exponential (no software pipeline)
   // bounded-score kernel with measured bounds: p = exp2(s - head_shift[h]); rows whose sum falls below ntok * 2^-14 (all their
   // scores far below the head's bound: the fp16 probabilities would be subnormal) flag their (tile, head pair) for an exact redo
   const float* head_shift;      // [H] or null (no shift)
   int* redo_count; int* redo_list; int* redo_flag;      // device work list filled by the bounded-score kernel (or null)
   // online-softmax kernel in list mode: items come from a device work list written by an earlier launch
   const int* work_count; const int* work_list;
-  unsigned long long* timers;   // k_attn_fast<.., true>: phase clocks of CTA 0 (see hy3d_debug_timers)
 };
 
 struct AttnBars {                          // mbarrier addresses (shared window), per stream a
@@ -192,17 +191,10 @@ __device__ __forceinline__ void attn_mma(const AttnTC& g, const AttnBars& B, uin
   uint64_t ring_d = make_desc_sw128(smem_u32(smem + 2 * TILE_BYTES + (sh ? 0 : a * ATT_SLOTS * TILE_BYTES)));
   asm volatile("" : "+r"(d_s), "+r"(d_o), "+r"(a_p), "+l"(qd), "+l"(ring_d));
   int s = 0; uint32_t ph = 0, qph = 0, sph = 0, pph = 0;
-  // instrumented launches (hy3d_debug_timers): cycles this warp waits for 0 K tile, 1 S buffer free, 2 V tile, 3 P stored
-  const bool tmr = g.timers != nullptr && blockIdx.x == 0;
-  long long tw[4] = {0, 0, 0, 0}, t0 = 0;
-  auto tick = [&](int i) { if (tmr) { const long long t_ = clock64(); tw[i] += t_ - t0; t0 = t_; } };
   auto issue_s = [&]() {
     const uint32_t full = sh ? B.kvfull_sh(s) : B.kvfull(a, s), empty = sh ? B.kvempty_sh(s) : B.kvempty(a, s);
-    if (tmr) t0 = clock64();
     mbar_wait(full, ph);
-    tick(0);
     mbar_wait(B.sempty(a), sph ^ 1); sph ^= 1;
-    tick(1);
     fence_after_sync();
     const uint64_t bd = ring_d + (uint64_t)(s * (TILE_BYTES / 16));
     if (elect_one()) {
@@ -216,11 +208,8 @@ __device__ __forceinline__ void attn_mma(const AttnTC& g, const AttnBars& B, uin
   };
   auto issue_pv = [&](int j) {
     const uint32_t full = sh ? B.kvfull_sh(s) : B.kvfull(a, s), empty = sh ? B.kvempty_sh(s) : B.kvempty(a, s);
-    if (tmr) t0 = clock64();
     mbar_wait(full, ph);
-    tick(2);
     mbar_wait(B.pfull(a), pph); pph ^= 1;
-    tick(3);
     fence_after_sync();
     const uint64_t bd = ring_d + (uint64_t)(s * (TILE_BYTES / 16));
     if (elect_one()) {
@@ -243,12 +232,10 @@ __device__ __forceinline__ void attn_mma(const AttnTC& g, const AttnBars& B, uin
       issue_pv(j);
     }
   }
-  if (tmr && (threadIdx.x & 31) == 0)
-    for (int i = 0; i < 4; ++i) atomicAdd(&g.timers[16 + a * 4 + i], (unsigned long long)tw[i]);
 }
 
 // exp2 on the FMA/ALU pipes (Cody-Waite split + degree-3 minimax on [-0.5, 0.5], max rel. error 1.6e-4, below the
-// fp16 rounding of the stored probability): takes kPoly of every 8 exponentials off the SFU.
+// fp16 rounding of the stored probability): takes some of the exponentials off the SFU.
 __device__ __forceinline__ float exp2_poly(float x) {
   x = fmaxf(x, -126.f);
   const float t = x + 12582912.f;                 // round to nearest integer in the low mantissa bits
@@ -293,7 +280,6 @@ __device__ __forceinline__ void exp2_poly2(float x0, float x1, float& p0, float&
 // ------------------------------------------------------------------------------------------
 // Bounded scores: no running maximum, two threads per query row.
 // ------------------------------------------------------------------------------------------
-template <int kPoly, bool kTimers>
 __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
   extern __shared__ __align__(1024) uint8_t smem_raw[];
   uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -328,8 +314,6 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
     int col0 = hh * 64;                                  // first token column of this thread inside a KV tile
     asm volatile("" : "+r"(bar_sfull), "+r"(bar_sempty), "+r"(bar_pfull), "+r"(bar_pvdone), "+r"(ts_), "+r"(tp_), "+r"(lane0), "+r"(col0));
     uint32_t sfull_ph = 0, pv_ph = 0;
-    long long tk0 = 0, tk[6] = {0, 0, 0, 0, 0, 0};
-#define HY3D_TICK(i) if constexpr (kTimers) { const long long t_ = clock64(); tk[i] += t_ - tk0; tk0 = t_; }
     for (int item = blockIdx.x; item < nitems; item += gridDim.x) {
       const AttnItem wi = attn_item(g, item, a);
       const int qt = wi.qt, h = wi.h;
@@ -337,7 +321,6 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
       uint64_t l2 = 0ull;                                // packed (even columns, odd columns) row sums: one FADD2 per pair
       const float cshift = g.head_shift ? g.head_shift[h] : 0.f;       // 0 unless the head's measured score bound exceeds 15.9
       const uint64_t cshift2 = pack_f2(cshift, cshift);
-      if constexpr (kTimers) tk0 = clock64();
       // Every barrier round trip of these warps queues behind the MUFU instructions already in the SM's MIO pipe (the
       // kernel's bottleneck): a wait costs ~450 clk even when the barrier completed long ago (instrumented: wait S 497,
       // wait PV 482 clk per tile of 2840).  So the two MMA-completion barriers are PROBED in the middle of the
@@ -347,18 +330,12 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
         if (!s_ready) mbar_wait(bar_sfull, sfull_ph);
         sfull_ph ^= 1;
         fence_after_sync();
-        HY3D_TICK(0)
         // software pipeline over the two 32-column halves of this thread's 64 scores: the second tcgen05.ld is in flight
         // while the first half's exponentials run (one TMEM round trip per tile off the stream's serial chain)
         uint32_t sv[64];
         HY3D_TMEM_LD32(ts_, sv);
-        if (g.no_pipe) {                                 // (experiment bit 0x200: both halves up front, S released before any exponential)
-          HY3D_TMEM_LD32(ts_ + 32, (sv + 32)); tmem_wait_ld();
-          fence_before_sync();
-          __syncwarp();
-          if (lane0) mbar_arrive(bar_sempty);
-        } else { tmem_wait_ld(); HY3D_TMEM_LD32(ts_ + 32, (sv + 32)); }
-        HY3D_TICK(1)
+        tmem_wait_ld();
+        HY3D_TMEM_LD32(ts_ + 32, (sv + 32));
         const int valid = ntok - j * 128 - col0;     // columns >= valid are padding tokens (last tile of a ragged count)
         bool pv_ok = j == 0, s_ok = false;
         if (cshift != 0.f) {                           // (warp-uniform) s - c_h: one FADD2 per pair, only for heads that need it
@@ -379,7 +356,7 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
               }
               const float x0 = __uint_as_float(sv[2 * i]), x1 = __uint_as_float(sv[2 * i + 1]);
               float p0, p1;
-              if (pair_on_fma<kPoly>(i)) exp2_poly2(x0, x1, p0, p1);
+              if (pair_on_fma<ATT_POLY_PAIRS>(i)) exp2_poly2(x0, x1, p0, p1);
               else { p0 = ex2(x0); p1 = ex2(x1); }
               l2 = add_f2(l2, pack_f2(p0, p1));
               sv[i] = pack_h2(p0, p1);
@@ -395,12 +372,10 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
           }
         };
         exp_pairs(0, 16);
-        if (!g.no_pipe) {
-          HY3D_TMEM_WAIT_LD32((sv + 32));              // second half has landed (tied to its registers)
-          fence_before_sync();
-          __syncwarp();
-          if (lane0) mbar_arrive(bar_sempty);          // S is in registers: the next S MMA may overwrite it
-        }
+        HY3D_TMEM_WAIT_LD32((sv + 32));                // second half has landed (tied to its registers)
+        fence_before_sync();
+        __syncwarp();
+        if (lane0) mbar_arrive(bar_sempty);            // S is in registers: the next S MMA may overwrite it
         if (cshift != 0.f) {
 #pragma unroll
           for (int i = 16; i < 32; ++i) {
@@ -410,16 +385,13 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
           }
         }
         exp_pairs(16, 32);
-        HY3D_TICK(2)
         if (j > 0) { if (!pv_ok) mbar_wait(bar_pvdone, pv_ph); pv_ph ^= 1; }   // PV(j-1) has consumed the previous P
         s_ready = s_ok;
-        HY3D_TICK(3)
         HY3D_TMEM_ST32(tp_, sv);
         tmem_wait_st();
         fence_before_sync();
         __syncwarp();
         if (lane0) mbar_arrive(bar_pfull);
-        HY3D_TICK(4)
       }
       // ---- finalize: row sums of the two column halves through shared memory, O / l -> fp16 tile (q-tile, head) ----
       float* ls = lsum + a * 256;
@@ -457,16 +429,7 @@ __global__ void __launch_bounds__(ATT_FAST_THREADS, 1) k_attn_fast(AttnTC g) {
       }
       fence_before_sync();
       asm volatile("bar.sync %0, 256;" ::"r"(1 + a) : "memory");   // ls[] is reused by the next item
-      HY3D_TICK(5)
-      if constexpr (kTimers) {
-        if (g.timers && lane == 0 && q == 0 && hh == 0 && blockIdx.x == 0) {
-#pragma unroll
-          for (int i = 0; i < 6; ++i) { atomicAdd(&g.timers[a * 8 + i], (unsigned long long)tk[i]); tk[i] = 0; }
-          atomicAdd(&g.timers[a * 8 + 7], (unsigned long long)nkv);
-        }
-      }
     }
-#undef HY3D_TICK
   }
   fence_before_sync();
   __syncthreads();

@@ -42,9 +42,9 @@ struct DecoderWeights {
   const float *fc_w, *fc_b, *mp_w, *mp_b, *lnp_w, *lnp_b, *out_w, *out_b;
   // tcgen05 operand images (decoder_tc.cu)
   DevBuf tc;
-  const __half *t_qp, *t_cq, *t_cproj, *t_fc, *t_mp;      // B tiles
+  const __half *t_qp, *t_fc, *t_mp;                       // B tiles
   DevBuf fold;                        // LayerNorm-folded epilogue constants (decoder_tc.cu)
-  const float *cs_q, *bb_q, *cs_fc, *bb_fc, *dotw, *c12;
+  const float *bb_q, *cs_fc, *bb_fc, *dotw, *c12;
   const __half *t_ckv3, *t_lp3;                           // c_kv (ln_2 folded, [k | v] rows) and latents_proj, 3-term split
   const float *cs_kv, *bb_kv;
   const __half* t_cqx = nullptr;                         // c_q . query_proj collapsed into one K = 192 image (x0 never formed)
@@ -115,7 +115,8 @@ struct DmcState {                     // dual marching cubes (dmc.cu): hy3d_dmc_
   DevBuf bits, rowcnt, rowoff, stats, rec;
 };
 
-// Per-kernel-family device timing with CUDA events on the launch stream (bench.py roofline).
+// Per-kernel-family device timing with CUDA events on the launch stream (bench.py roofline).  The numbering is part of the
+// C-ABI (hy3d_profile_read): FAM_GEMM_QPROJ and FAM_LN keep their slots although no launch records them any more.
 enum { FAM_EMBED = 0, FAM_GEMM_QPROJ, FAM_LN, FAM_GEMM_CQ, FAM_ATTN, FAM_GEMM_CPROJ, FAM_GEMM_FC, FAM_GEMM_MLP, FAM_HEAD,
        FAM_MC_BITS, FAM_MC_ROWCOUNT, FAM_MC_SCAN, FAM_MC_EMIT, FAM_OCTREE, FAM_KV, FAM_SELECT, FAM_COUNT };
 struct ProfRec { int fam; cudaEvent_t e0, e1; };
@@ -147,21 +148,10 @@ struct hy3d_ctx {
   Prof prof;
   // per-context launch state of the tcgen05 path (was function-local statics: one context per thread and device)
   void* tmap_encode = nullptr;        // cuTensorMapEncodeTiled entry point
-  int l2_promo = -1;                  // HY3D_L2PROMO
   int gemm_max_clusters[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // co-resident CTA pairs per GEMM epilogue variant
   std::vector<float> axis_host;       // last per-axis coordinate tables uploaded to ws[11] (skips the upload when unchanged)
-  // diagnostics: per-stage activations of the last decoded chunk (hy3d_debug_retain / hy3d_debug_fetch)
-  int attn_poly = 2;                  // bounded-score attention kernel: PAIRS of every 8 pairs of exponentials evaluated as packed polynomials on the FMA pipe (HY3D_ATTN_POLY: 0 none, 1 .. 6 = that many pairs, 8 = all; default 2 = a quarter of the exponentials, re-tuned after the loop overhead went away: 2 and 3 tie, 4 is 3 % slower, 0 is 11 % slower; any other value = default)
-  int debug_retain = 0;
-  long long chunk_points = 262144;    // decoder chunk (HY3D_CHUNK; 131072 measured 1 % slower, 32768 7 % slower): activations of one chunk are what the stages hand over through L2 / HBM
-  int xbits = 0;                      // HY3D_DBG: experiment bits for tools/gpu_chain_bench.py (results are garbage when set)
-  DevBuf dbg[8];
-  int dbg_layout[8] = {0, 0, 0, 0, 0, 0, 0, 0};   // 0 row-major fp32, 1 R32, 2 T16
-  long long dbg_rows = 0;
-  int dbg_width[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  int force_online_softmax = 0;       // hy3d_debug_force_online_softmax: tests run the online-softmax kernel as a reference
 };
-// stage ids: 0 x0, 1 ln_1(x0), 2 q (after q_norm), 3 attention out, 4 x1, 5 ln_3(x1), 6 mlp hidden, 7 x2
-int hy3d_debug_keep(hy3d_ctx* ctx, int stage, const void* src, size_t bytes, int layout, long long rows, int width);
 
 int hy3d_fail(hy3d_ctx* ctx, int code, const char* fmt, ...);
 // tcgen05 watchdog (tc_ptx.cuh): enqueue the read-back of the record before a stream synchronisation that happens anyway,

@@ -285,9 +285,7 @@ int hy3d_decode_simt(hy3d_ctx* ctx, const QuerySource& src_in, long long n, floa
     else src.index += p0;
     k_embed_qproj<<<(unsigned)ceil_div64(P, EQ_PTS), 256, 0, ctx->stream>>>(src, P, w.F, w.include_pi, w.qp_w, w.qp_b, W, x);
     HY3D_LAUNCH_CHECK(ctx);
-    if (int rc = hy3d_debug_keep(ctx, 0, x, (size_t)P * W * 4, 0, P, W)) return rc;
     if (int rc = layernorm(ctx, x, P, W, W, w.ln1_w, w.ln1_b, 1e-6f, 1.f, t, W)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 1, t, (size_t)P * W * 4, 0, P, W)) return rc;
     {   // q = c_q(ln_1(x))   (written to a, then head-normed in place)
       GemmArgs g{};
       g.A = t; g.lda = W; g.B = w.cq_w; g.ldb = W; g.C = a; g.ldc = W; g.bias = w.cq_b; g.M = P; g.N = W; g.K = W; g.alpha = 1.f;
@@ -295,7 +293,6 @@ int hy3d_decode_simt(hy3d_ctx* ctx, const QuerySource& src_in, long long n, floa
     }
     if (w.qk_norm)
       if (int rc = layernorm(ctx, a, P * H, D, D, w.qn_w, w.qn_b, 1e-6f, 1.f, a, D)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 2, a, (size_t)P * W * 4, 0, P, W)) return rc;
     {   // scores[h] = q_h k_h^T / sqrt(D)
       GemmArgs g{};
       g.A = a; g.lda = W; g.sA = D; g.B = ctx->kv.k32.as<float>(); g.ldb = D; g.sB = (long long)M * D;
@@ -310,30 +307,25 @@ int hy3d_decode_simt(hy3d_ctx* ctx, const QuerySource& src_in, long long n, floa
       g.C = t; g.ldc = W; g.sC = D; g.M = P; g.N = D; g.K = M; g.alpha = 1.f;
       if (int rc = sgemm(ctx, g, H)) return rc;
     }
-    if (int rc = hy3d_debug_keep(ctx, 3, t, (size_t)P * W * 4, 0, P, W)) return rc;
     {   // x1 = x0 + c_proj(attn)
       GemmArgs g{};
       g.A = t; g.lda = W; g.B = w.cproj_w; g.ldb = W; g.C = x; g.ldc = W; g.bias = w.cproj_b; g.resid = x; g.ldr = W;
       g.M = P; g.N = W; g.K = W; g.alpha = 1.f;
       if (int rc = sgemm(ctx, g, 1)) return rc;
     }
-    if (int rc = hy3d_debug_keep(ctx, 4, x, (size_t)P * W * 4, 0, P, W)) return rc;
     if (int rc = layernorm(ctx, x, P, W, W, w.ln3_w, w.ln3_b, 1e-6f, 1.f, t, W)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 5, t, (size_t)P * W * 4, 0, P, W)) return rc;
     {   // h = gelu(c_fc(ln_3 x1))
       GemmArgs g{};
       g.A = t; g.lda = W; g.B = w.fc_w; g.ldb = W; g.C = h; g.ldc = (long long)W * R; g.bias = w.fc_b; g.gelu = 1;
       g.M = P; g.N = W * R; g.K = W; g.alpha = 1.f;
       if (int rc = sgemm(ctx, g, 1)) return rc;
     }
-    if (int rc = hy3d_debug_keep(ctx, 6, h, (size_t)P * W * R * 4, 0, P, W * R)) return rc;
     {   // x2 = x1 + c_proj(h)
       GemmArgs g{};
       g.A = h; g.lda = (long long)W * R; g.B = w.mp_w; g.ldb = (long long)W * R; g.C = x; g.ldc = W; g.bias = w.mp_b;
       g.resid = x; g.ldr = W; g.M = P; g.N = W; g.K = W * R; g.alpha = 1.f;
       if (int rc = sgemm(ctx, g, 1)) return rc;
     }
-    if (int rc = hy3d_debug_keep(ctx, 7, x, (size_t)P * W * 4, 0, P, W)) return rc;
     float* outp = d_out + (out_mode == 0 ? p0 : 0);
     k_head_out<<<(unsigned)ceil_div64(P, 8), 256, 0, ctx->stream>>>(x, P, W, w.ln_post ? w.lnp_w : nullptr, w.lnp_b, w.out_w,
                                                                    w.out_b, src, outp, out_mode);

@@ -11,15 +11,15 @@
 //                                                          contiguous per warp instruction)
 //   K      fp16 [group][head][M/128][128 tok x 64, SW128]      V^T fp16 [group][head][M/128][2][64 d x 64 tok, SW128]
 //
-// Stage chain per chunk of 131072 points (one launch each, activations through HBM/L2; the chain is
+// Stage chain per chunk of 262144 points (one launch each, activations through HBM/L2; the chain is
 // compute-bound: ~30 KB/point of traffic vs 33.7 MFLOP/point).  The three LayerNorms never run as kernels: ln_1 / ln_3
 // are folded into the consuming GEMM (raw operand, gamma in the weights, per-row statistics from the producer's
-// epilogue), ln_post into the head:
-//   k_embed_tc       Fourier features, fp16 hi/lo split                          -> T16 [., 3]
-//   k_gemm_tc<X0>    query_proj (3-term split fp16 = ~fp32)                       -> R32 x0, T16 raw x0, row stats
-//   k_gemm_tc<Q>     c_q (ln_1 folded), per-head q_norm, * scale * log2e          -> T16 q (k-block == head)
+// epilogue or, for ln_1, from the embed kernel), ln_post into the head.  x0 = query_proj(e) is never formed:
+//   k_embed_tc       Fourier features, fp16 hi/lo split; ln_1 statistics of x0   -> T16 [., 3], row (mean, rstd)
+//   k_gemm_tc<Q>     c_q . query_proj collapsed (K = 192, ln_1 folded), per-head q_norm, * scale * log2e
+//                                                                                -> T16 q (k-block == head)
 //   k_attn_fast / k_attn_tc   softmax(q k^T) v, 2 heads in flight per CTA (attention_tc.cuh)  -> T16
-//   k_gemm_tc<RES>   c_proj + residual                                           -> R32 x1, T16 raw x1, row stats
+//   k_gemm_tc<RES>   x0 + c_proj: [attn | e] [W_o | W_qp]^T (K = W + 192)          -> R32 x1, T16 raw x1, row stats
 //   k_gemm_tc<GELU>  c_fc (ln_3 folded) + erf-GELU                                -> T16 h
 //   k_gemm_tc<RES>   mlp.c_proj + residual: only row stats + dot with gamma_post * w_out leave the kernel
 //   k_head_final     [ln_post] + output_proj from those statistics               -> logits (dense or scattered)
@@ -31,7 +31,6 @@
 
 using namespace tc;
 
-__device__ unsigned long long hy3d_tm[32];   // phase clocks of the instrumented attention kernel (hy3d_debug_timers)
 namespace {
 
 constexpr int TILE_M = 128;
@@ -72,7 +71,6 @@ struct GemmTC {
   uint8_t* Kout; uint8_t* Vout; const float* kn_w; const float* kn_b; int nkv; int Wq;
   int part0;             // 0: columns [q | k | v] (latent transformer); 1: columns [k | v] (decoder c_kv)
   float* K32; float* V32T; int Mtok;   // optional fp32 copies k [H, Mtok, 64], v^T [H, 64, Mtok] (FlashVDM selection); rows >= Mtok are written as zeros
-  int dbg;               // HY3D_DBG experiment bits: 1 no epilogue, 2 no MMA, 4 no epilogue stores
 };
 
 // merge S partial (mean, M2) pairs of n_p samples each -> (mean, rstd)   (Chan et al., deterministic order)
@@ -196,7 +194,6 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
   uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(bars + 2 * GEMM_STAGES + 4);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-  const long long clk0 = (g.dbg & 8) ? clock64() : 0;
   if (threadIdx.x == 0) {
     for (int s = 0; s < GEMM_STAGES; ++s) { mbar_init(FULL(s), 1); mbar_init(EMPTY(s), GEMM_CL / 2); }
     for (int a = 0; a < 2; ++a) { mbar_init(TFULL(a), 1); mbar_init(TEMPTY(a), 32); }
@@ -250,35 +247,27 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const uint32_t idesc = make_idesc_f16(2 * TILE_M, BN);
     int s = 0; uint32_t ph = 0;
     int it = 0;
-    long long tw0 = 0, tw[3] = {0, 0, 0};          // (experiment bit 8) cycles: wait TEMPTY, wait FULL, issue
-    const bool tmr = (g.dbg & 8) && blockIdx.x == 0;
     for (int p = cid; p < npairs; p += ncl, ++it) {
       const int acc = it & 1;
       const uint32_t aph = (it >> 1) & 1;
-      if (tmr) tw0 = clock64();
       mbar_wait(TEMPTY(acc), aph ^ 1);
       fence_after_sync();
-      if (tmr) { const long long t_ = clock64(); tw[0] += t_ - tw0; tw0 = t_; }
       const uint32_t d = tmem + acc * BN;
       for (int kb = 0; kb < g.KB; ++kb) {
         mbar_wait(FULL(s), ph);
         fence_after_sync();
-        if (tmr) { const long long t_ = clock64(); tw[1] += t_ - tw0; tw0 = t_; }
         const uint64_t ad = make_desc_sw128(smem_u32(sA + s * TILE_BYTES));
         const uint64_t bd = make_desc_sw128(smem_u32(sB + s * TILE_BYTES));
         if (elect_one()) {
-          if (!(g.dbg & 2))
 #pragma unroll
-            for (int k = 0; k < 4; ++k) mma2_f16_ss(d, ad + 2 * k, bd + 2 * k, idesc, (kb | k) != 0);
+          for (int k = 0; k < 4; ++k) mma2_f16_ss(d, ad + 2 * k, bd + 2 * k, idesc, (kb | k) != 0);
           mma2_commit_multicast(EMPTY(s), mask_all);
           if (kb == g.KB - 1) mma2_commit_multicast(TFULL(acc), mask_pair);
         }
         __syncwarp();
-        if (tmr) { const long long t_ = clock64(); tw[2] += t_ - tw0; tw0 = t_; }
         if (++s == GEMM_STAGES) { s = 0; ph ^= 1; }
       }
     }
-    if (tmr && lane == 0) { for (int i = 0; i < 3; ++i) atomicAdd(&hy3d_tm[16 + i], (unsigned long long)tw[i]); atomicAdd(&hy3d_tm[19], (unsigned long long)it); }
   } else if (warp >= 4) {
     // ---------------- epilogue: 16 warps = 4 TMEM lane quadrants x 4 column quarters of 64 ----------------
     // (four warps per scheduler: the TMEM-load -> constants -> math -> store chain of one warp hides behind the others)
@@ -286,17 +275,13 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
     const int cq = (warp - 4) >> 2;         // 64-column quarter of the 256-wide tile
     const int r = q * 32 + lane;            // row inside the tile
     int it = 0;
-    long long te0 = 0, te[2] = {0, 0};              // (experiment bit 8) cycles: wait TFULL, work
-    const bool tmr = (g.dbg & 8) && blockIdx.x == 0 && warp == 4;
     for (int p = cid; p < npairs; p += ncl, ++it) {
       const int mb = GEMM_CL * (p / g.Nb) + crank, nb = p % g.Nb;
       const int acc = it & 1;
       const uint32_t aph = (it >> 1) & 1;
-      if (tmr) { const long long t_ = clock64(); if (it) te[1] += t_ - te0; te0 = t_; }
       mbar_wait(TFULL(acc), aph);
       fence_after_sync();
-      if (tmr) { const long long t_ = clock64(); te[0] += t_ - te0; te0 = t_; }
-      if ((g.dbg & 1) || mb >= g.Mb) {
+      if (mb >= g.Mb) {
         fence_before_sync(); __syncwarp();
         if (lane == 0) { if (rank == 0) mbar_arrive(TEMPTY(acc)); else mbar_arrive_remote(TEMPTY(acc), crank & ~1); }
         continue;
@@ -391,12 +376,7 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
 #pragma unroll
             for (int i = 0; i < 32; ++i) x[i] = 0.f;
           }
-          if (g.dbg & 4) {
-            float acc_ = 0.f;
-#pragma unroll
-            for (int i = 0; i < 32; ++i) acc_ += x[i];
-            if (acc_ == 123.456f) g.Tout[0] = 1;
-          } else if constexpr (EPI == EPI_QF32) {
+          if constexpr (EPI == EPI_QF32) {
             float4* o = reinterpret_cast<float4*>(g.Fout + (size_t)row * g.N + c0 + ch * 32);
 #pragma unroll
             for (int i4 = 0; i4 < 8; ++i4) o[i4] = make_float4(x[4 * i4], x[4 * i4 + 1], x[4 * i4 + 2], x[4 * i4 + 3]);
@@ -440,12 +420,7 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
             }
             const int KBn = g.N / 64;
             uint8_t* tile = g.Tout + ((size_t)mb * (g.split_out ? 3 : 1) * KBn + (c >> 6)) * TILE_BYTES;
-            if (g.dbg & 4) {
-              float acc_ = 0.f;
-#pragma unroll
-              for (int i = 0; i < 32; ++i) acc_ += x[i];
-              if (acc_ == 123.456f) g.Tout[0] = 1;
-            } else if (g.split_out) {
+            if (g.split_out) {
 #pragma unroll
               for (int c16 = 0; c16 < 4; ++c16)
                 store_t16_split(tile, tile + (size_t)KBn * TILE_BYTES, tile + (size_t)2 * KBn * TILE_BYTES, r, ch * 4 + c16, x + 8 * c16);
@@ -466,9 +441,9 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
                 o.x += rr.x; o.y += rr.y; o.z += rr.z; o.w += rr.w;
                 x[4 * i4] = o.x; x[4 * i4 + 1] = o.y; x[4 * i4 + 2] = o.z; x[4 * i4 + 3] = o.w;
               }
-              if (g.Rout && !(g.dbg & 4)) reinterpret_cast<float4*>(g.Rout)[idx] = o;
+              if (g.Rout) reinterpret_cast<float4*>(g.Rout)[idx] = o;
             }
-            if (g.Tcopy && !(g.dbg & 4)) {
+            if (g.Tcopy) {
               const int KBn = g.N / 64;
               uint8_t* tile = g.Tcopy + ((size_t)mb * (g.split_out ? 3 : 1) * KBn + (c >> 6)) * TILE_BYTES;
               if (g.split_out) {
@@ -516,13 +491,11 @@ k_gemm_tc(GemmTC g, const __grid_constant__ CUtensorMap tmA, const __grid_consta
       __syncwarp();
       if (lane == 0) { if (rank == 0) mbar_arrive(TEMPTY(acc)); else mbar_arrive_remote(TEMPTY(acc), crank & ~1); }
     }
-    if (tmr && lane == 0) { te[1] += clock64() - te0; atomicAdd(&hy3d_tm[20], (unsigned long long)te[0]); atomicAdd(&hy3d_tm[21], (unsigned long long)te[1]); }
   }
   if (warp >= 4 && (warp & 3) == 0 && lane == 0) bulk_wait_all();   // staged output tiles have reached global memory
   fence_before_sync();
   cluster_sync();                      // the peer may still be signalling this CTA's barriers
   if (warp == 2) tmem_dealloc2(tmem, 512);
-  if ((g.dbg & 8) && threadIdx.x == 0 && blockIdx.x == 0) atomicAdd(&hy3d_tm[24 + EPI], (unsigned long long)(clock64() - clk0));   // SM cycles of this launch
 }
 
 constexpr size_t GEMM_SMEM = 1024 + GEMM_STAGES * 2 * TILE_BYTES + ST_PER_TILE * TILE_BYTES + 256;
@@ -803,8 +776,10 @@ __global__ void __launch_bounds__(256) k_qstats_consts(const float* __restrict__
 // ---- operand image builders ----------------------------------------------------------------
 // fp32 row-major W[N, K] (ld = ldw) -> B16 tiles.  mode 0: plain.  mode 1: query_proj split:
 // K_out = 192 = [W_hi | W_hi | W_lo] over the first E columns (zero padded to 64).  mode 2: the same
-// 3-term split for a full [N, K/3] matrix.
-__global__ void k_build_b16(const float* __restrict__ Wsrc, int N, int K, int ldw, int mode, int E, uint8_t* __restrict__ out) {
+// 3-term split for a full [N, K/3] matrix.  kbs: k-blocks per 256-row block of `out` (0 = K / 64; more when the image is
+// one part of a K-concatenated operand).
+__global__ void k_build_b16(const float* __restrict__ Wsrc, int N, int K, int ldw, int mode, int E, uint8_t* __restrict__ out,
+                            int kbs = 0) {
   const int KB = K / 64;
   long long t = (long long)blockIdx.x * blockDim.x + threadIdx.x;    // one 16-byte chunk per thread
   long long total = (long long)N * (K / 8);
@@ -830,7 +805,7 @@ __global__ void k_build_b16(const float* __restrict__ Wsrc, int N, int K, int ld
     }
     v[i] = w;
   }
-  uint8_t* tile = out + ((size_t)(n / BN) * KB + kb) * BTILE_BYTES;
+  uint8_t* tile = out + ((size_t)(n / BN) * (kbs ? kbs : KB) + kb) * BTILE_BYTES;
   store_t16_chunk(tile, n % BN, c16, v);
 }
 
@@ -880,12 +855,9 @@ int make_rows_map(hy3d_ctx* ctx, CUtensorMap* m, const void* base, uint64_t rows
   const cuuint64_t strides[1] = {2048};
   const cuuint32_t box[2] = {256, (cuuint32_t)box_rows};     // 8 rows of 2 KB = one 16 KB tile (4 = half of it)
   const cuuint32_t estr[2] = {1, 1};
-  if (ctx->l2_promo < 0) { const char* e = getenv("HY3D_L2PROMO"); ctx->l2_promo = e ? atoi(e) : 3; }   // 0 none, 1 64 B, 2 128 B, 3 256 B (default)
-  const int promo = ctx->l2_promo;
-  const CUtensorMapL2promotion pr = promo == 0 ? CU_TENSOR_MAP_L2_PROMOTION_NONE : promo == 1 ? CU_TENSOR_MAP_L2_PROMOTION_L2_64B
-                                  : promo == 2 ? CU_TENSOR_MAP_L2_PROMOTION_L2_128B : CU_TENSOR_MAP_L2_PROMOTION_L2_256B;
+  // 256 B L2 promotion, the widest: every box row is 2 KB of contiguous bytes that the copy reads whole
   const CUresult r = encode(m, CU_TENSOR_MAP_DATA_TYPE_UINT64, 2, const_cast<void*>(base), dims, strides, box, estr, CU_TENSOR_MAP_INTERLEAVE_NONE,
-                            CU_TENSOR_MAP_SWIZZLE_NONE, pr, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+                            CU_TENSOR_MAP_SWIZZLE_NONE, CU_TENSOR_MAP_L2_PROMOTION_L2_256B, CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
   if (r != CUDA_SUCCESS) return hy3d_fail(ctx, HY3D_ERR_CUDA, "cuTensorMapEncodeTiled failed (%d)", (int)r);
   return 0;
 }
@@ -915,7 +887,7 @@ int launch_gemm(hy3d_ctx* ctx, const GemmTC& g, int fam) {
   const int pairs = ((g.Mb + GEMM_CL - 1) / GEMM_CL) * g.Nb;        // one group of GEMM_CL vertically adjacent tiles per cluster iteration
   const int grid = GEMM_CL * (pairs < max_clusters ? pairs : max_clusters);
   HY3D_PROF(ctx, fam);
-  GemmTC gd = g; gd.dbg = ctx->xbits & 15;
+  GemmTC gd = g;
   if (g.st_in) {
     const long long rows = (long long)g.Mb * TILE_M;
     HY3D_CUDA(ctx, ctx->ln_mr.reserve((size_t)rows * sizeof(float2)));
@@ -934,8 +906,6 @@ int launch_gemm(hy3d_ctx* ctx, const GemmTC& g, int fam) {
 }
 
 // Attention launch: the bounded-score kernel when `fast` (see attention_tc.cuh), else the online-softmax kernel.
-// ctx->attn_poly = how many of every 8 exponentials run on the FMA pipe; ctx->xbits & 0x20 forces the general kernel,
-// 0x40 runs the instrumented fast kernel (hy3d_debug_timers).
 template <class K>
 int launch_attn_kernel(hy3d_ctx* ctx, K kern, const AttnTC& a, int threads) {
   HY3D_CUDA(ctx, cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)ATT_SMEM));
@@ -945,7 +915,7 @@ int launch_attn_kernel(hy3d_ctx* ctx, K kern, const AttnTC& a, int threads) {
   return 0;
 }
 int launch_attn(hy3d_ctx* ctx, AttnTC a, bool fast, int fam, bool shifted = false) {
-  if (ctx->xbits & 0x20) fast = false;
+  if (ctx->force_online_softmax) fast = false;
   KVState& kv = ctx->kv;
   if (fast && shifted) {                                   // decoder attention with measured per-head bounds (k_head_shift)
     const size_t items = (size_t)a.Pb * (a.H / 2);
@@ -956,30 +926,8 @@ int launch_attn(hy3d_ctx* ctx, AttnTC a, bool fast, int fam, bool shifted = fals
   }
   HY3D_PROF(ctx, fam);
   // one K/V set for all query tiles (no per-tile KV groups): pairs of query tiles share every K/V tile they stream
-  a.share_kv = (a.tile_group == nullptr && !(ctx->xbits & 0x100)) ? 1 : 0;
-  a.no_pipe = (ctx->xbits & 0x200) ? 1 : 0;
-  int rc = 0;
-  if (fast) {
-    if (ctx->xbits & 0x40) {
-      void* tm = nullptr;
-      HY3D_CUDA(ctx, cudaGetSymbolAddress(&tm, hy3d_tm));
-      a.timers = reinterpret_cast<unsigned long long*>(tm);
-      rc = launch_attn_kernel(ctx, k_attn_fast<2, true>, a, ATT_FAST_THREADS);
-    } else {
-      switch (ctx->attn_poly) {            // pairs of every 8 whose exponentials run as packed polynomials on the FMA pipe
-        case 0: rc = launch_attn_kernel(ctx, k_attn_fast<0, false>, a, ATT_FAST_THREADS); break;
-        case 1: rc = launch_attn_kernel(ctx, k_attn_fast<1, false>, a, ATT_FAST_THREADS); break;
-        case 4: rc = launch_attn_kernel(ctx, k_attn_fast<4, false>, a, ATT_FAST_THREADS); break;
-        case 3: rc = launch_attn_kernel(ctx, k_attn_fast<3, false>, a, ATT_FAST_THREADS); break;
-        case 5: rc = launch_attn_kernel(ctx, k_attn_fast<5, false>, a, ATT_FAST_THREADS); break;
-        case 6: rc = launch_attn_kernel(ctx, k_attn_fast<6, false>, a, ATT_FAST_THREADS); break;
-        case 8: rc = launch_attn_kernel(ctx, k_attn_fast<8, false>, a, ATT_FAST_THREADS); break;
-        default: rc = launch_attn_kernel(ctx, k_attn_fast<2, false>, a, ATT_FAST_THREADS); break;
-      }
-    }
-  } else {
-    rc = launch_attn_kernel(ctx, k_attn_tc<0>, a, ATT_THREADS);
-  }
+  a.share_kv = a.tile_group == nullptr ? 1 : 0;
+  const int rc = fast ? launch_attn_kernel(ctx, k_attn_fast, a, ATT_FAST_THREADS) : launch_attn_kernel(ctx, k_attn_tc<0>, a, ATT_THREADS);
   if (rc) return rc;
   HY3D_LAUNCH_CHECK(ctx);
   if (fast && shifted) {
@@ -1057,31 +1005,28 @@ int hy3d_tc_prepare_weights(hy3d_ctx* ctx) {
     return 0;
   }
   const size_t W = w.W, R = w.R;
-  const size_t n_qp = W * 192, n_cq = W * W, n_cp = W * W, n_fc = R * W * W, n_mp = R * W * W, n_cq3 = 3 * W * W;
+  const size_t n_qp = W * 192, n_fc = R * W * W, n_mp = R * W * W, n_cq3 = 3 * W * W;
   const size_t n_ckv3 = 2 * W * 3 * W, n_lp3 = w.has_latents_proj ? W * 3 * (size_t)w.LW : 0;
   const size_t n_cpx = W * (W + 192);                               // [c_proj | query_proj split] concatenated along K
   const size_t n_cqx = W * 192;                                     // c_q . query_proj collapsed: [Wc_hi | Wc_hi | Wc_lo]
-  HY3D_CUDA(ctx, w.tc.reserve((n_qp + n_cq + n_cp + n_fc + n_mp + n_cq3 + n_ckv3 + n_lp3 + n_cpx + n_cqx) * 2));
-  __half* base = w.tc.as<__half>();
-  __half* p_qp = base; __half* p_cq = p_qp + n_qp; __half* p_cp = p_cq + n_cq; __half* p_fc = p_cp + n_cp; __half* p_mp = p_fc + n_fc;
-  auto build = [&](const float* src, int N, int K, int ldw, int mode, __half* dst) -> int {
+  HY3D_CUDA(ctx, w.tc.reserve((n_qp + n_fc + n_mp + n_cq3 + n_ckv3 + n_lp3 + n_cpx + n_cqx) * 2));
+  __half* p_qp = w.tc.as<__half>(); __half* p_fc = p_qp + n_qp; __half* p_mp = p_fc + n_fc; __half* p_cq3 = p_mp + n_mp;
+  __half* p_ckv3 = p_cq3 + n_cq3; __half* p_lp3 = p_ckv3 + n_ckv3; __half* p_cpx = p_lp3 + n_lp3; __half* p_cqx = p_cpx + n_cpx;
+  auto build = [&](const float* src, int N, int K, int ldw, int mode, __half* dst, int kbs = 0) -> int {
     long long total = (long long)N * (K / 8);
-    k_build_b16<<<(unsigned)ceil_div64(total, 256), 256, 0, ctx->stream>>>(src, N, K, ldw, mode, w.E, reinterpret_cast<uint8_t*>(dst));
+    k_build_b16<<<(unsigned)ceil_div64(total, 256), 256, 0, ctx->stream>>>(src, N, K, ldw, mode, w.E, reinterpret_cast<uint8_t*>(dst), kbs);
     HY3D_LAUNCH_CHECK(ctx);
     return 0;
   };
   // ln_1 folded into c_q, ln_3 into c_fc, ln_post into the head (see GemmTC)
   const size_t n_qs = 64 + 64 + 64 * 64 + 64 + W * 64 + W;          // wbar, hc, Gc, scalars, Wc rows (E + 1 <= 64 columns), exact cs
-  HY3D_CUDA(ctx, w.fold.reserve((W + W + R * W + R * W + W + 64 + 4 * W + W + n_qs) * sizeof(float)));
+  HY3D_CUDA(ctx, w.fold.reserve((W + R * W + R * W + W + 64 + 4 * W + W + n_qs) * sizeof(float)));
   HY3D_CUDA(ctx, ctx->ws[10].reserve(R * W * W * sizeof(float)));
   float* fb = w.fold.as<float>();
-  float* cs_q = fb; float* bb_q = cs_q + W; float* cs_fc = bb_q + W; float* bb_fc = cs_fc + R * W; float* dotw = bb_fc + R * W; float* c12 = dotw + W;
+  float* bb_q = fb; float* cs_fc = bb_q + W; float* bb_fc = cs_fc + R * W; float* dotw = bb_fc + R * W; float* c12 = dotw + W;
   float* Wf = ctx->ws[10].as<float>();
   if (int rc = build(w.qp_w, (int)W, 192, w.E, 1, p_qp)) return rc;
-  k_fold_ln<<<(unsigned)((W + 7) / 8), 256, 0, ctx->stream>>>(w.cq_w, w.ln1_w, w.ln1_b, w.cq_b, (int)W, (int)W, Wf, cs_q, bb_q, 0, 0);
-  HY3D_LAUNCH_CHECK(ctx);
-  if (int rc = build(Wf, (int)W, (int)W, (int)W, 0, p_cq)) return rc;
-  {   // collapsed c_q . query_proj (Wf still holds the gamma-folded c_q weight) + the closed-form ln_1 statistics of x0
+  {   // collapsed c_q . query_proj + the closed-form ln_1 statistics of x0
     float* qsb = c12 + 64 + 4 * W + W;
     float* wbar = qsb; float* hcv = wbar + 64; float* Gc = hcv + 64; float* scal = Gc + 64 * 64; float* Wc = scal + 64;
     float* cs_qx = Wc + W * 64;
@@ -1094,7 +1039,6 @@ int hy3d_tc_prepare_weights(hy3d_ctx* ctx) {
     HY3D_LAUNCH_CHECK(ctx);
     k_qstats_consts<<<1, 256, 0, ctx->stream>>>(w.qp_w, w.qp_b, (int)W, w.E, wbar, hcv, Gc, scal);
     HY3D_LAUNCH_CHECK(ctx);
-    __half* p_cqx = p_mp + n_mp + n_cq3 + n_ckv3 + n_lp3 + n_cpx;
     const int saveE = w.E;
     w.E = E1;                                                        // k_build_b16 mode 1 reads w.E valid columns
     const int rc = build(Wc, (int)W, 192, E1, 1, p_cqx);
@@ -1102,17 +1046,15 @@ int hy3d_tc_prepare_weights(hy3d_ctx* ctx) {
     if (rc) return rc;
     w.t_cqx = p_cqx; w.qs_wbar = wbar; w.qs_hc = hcv; w.qs_Gc = Gc; w.qs_scal = scal; w.cs_qx = cs_qx;
   }
-  if (int rc = build(w.cproj_w, (int)W, (int)W, (int)W, 0, p_cp)) return rc;
   k_fold_ln<<<(unsigned)((R * W + 7) / 8), 256, 0, ctx->stream>>>(w.fc_w, w.ln3_w, w.ln3_b, w.fc_b, (int)(R * W), (int)W, Wf, cs_fc, bb_fc, 0, 0);
   HY3D_LAUNCH_CHECK(ctx);
   if (int rc = build(Wf, (int)(R * W), (int)W, (int)W, 0, p_fc)) return rc;
   k_head_consts<<<1, 256, 0, ctx->stream>>>(w.ln_post ? w.lnp_w : nullptr, w.ln_post ? w.lnp_b : nullptr, w.out_w, w.out_b, (int)W, dotw, c12);
   HY3D_LAUNCH_CHECK(ctx);
-  w.cs_q = cs_q; w.bb_q = bb_q; w.cs_fc = cs_fc; w.bb_fc = bb_fc; w.dotw = dotw; w.c12 = c12;
+  w.bb_q = bb_q; w.cs_fc = cs_fc; w.bb_fc = bb_fc; w.dotw = dotw; w.c12 = c12;
   if (int rc = build(w.mp_w, (int)W, (int)(R * W), (int)(R * W), 0, p_mp)) return rc;
-  __half* p_cq3 = p_mp + n_mp;
   if (int rc = build(w.cq_w, (int)W, (int)(3 * W), (int)W, 2, p_cq3)) return rc;
-  w.t_qp = p_qp; w.t_cq = p_cq; w.t_cproj = p_cp; w.t_fc = p_fc; w.t_mp = p_mp; w.t_cq3 = p_cq3;
+  w.t_qp = p_qp; w.t_fc = p_fc; w.t_mp = p_mp; w.t_cq3 = p_cq3;
   w.attn_bound = INFINITY; w.attn_qbound = INFINITY; w.attn_fast = false;
   if (w.qk_norm) {
     if (int rc = attn_score_bound(ctx, w.qn_w, w.qn_b, w.kn_w, w.kn_b, &w.attn_bound, &w.attn_qbound)) return rc;
@@ -1127,7 +1069,6 @@ int hy3d_tc_prepare_weights(hy3d_ctx* ctx) {
   w.t_ckv3 = nullptr; w.t_lp3 = nullptr;
   if (w.LW % 64 == 0 && (!w.has_latents_proj || w.LW % 64 == 0)) {
     float* cs_kv = c12 + 64; float* bb_kv = cs_kv + 2 * W;
-    __half* p_ckv3 = p_cq3 + n_cq3; __half* p_lp3 = p_ckv3 + n_ckv3;
     k_fold_ln<<<(unsigned)((2 * W + 7) / 8), 256, 0, ctx->stream>>>(w.ckv_w, w.ln2_w, w.ln2_b, w.has_ckv_b ? w.ckv_b : nullptr, (int)(2 * W),
                                                                     (int)W, Wf, cs_kv, bb_kv, w.H, 1, 2);
     HY3D_LAUNCH_CHECK(ctx);
@@ -1137,17 +1078,12 @@ int hy3d_tc_prepare_weights(hy3d_ctx* ctx) {
     w.t_ckv3 = p_ckv3; w.t_lp3 = w.has_latents_proj ? p_lp3 : nullptr; w.cs_kv = cs_kv; w.bb_kv = bb_kv;
   }
   // x1 = x0 + c_proj(attn) + b  as ONE GEMM over K = W + 192: [attn | e_hi | e_lo | e_hi] [W_o | W_qp,hi | W_qp,hi | W_qp,lo]^T
-  // + (b_o + b_qp) — the fp32 x0 never travels through HBM.  Tile images are concatenated per 256-row block.
+  // + (b_o + b_qp) — the fp32 x0 never travels through HBM.  Per 256-row block the image holds the W / 64 k-blocks of c_proj,
+  // then the 3 of the query_proj split.
   {
-    __half* p_cpx = p_cq3 + n_cq3 + n_ckv3 + n_lp3;
-    const size_t kb_o = W / 64, kb_x = kb_o + 3;
-    for (size_t nb = 0; nb < W / BN; ++nb) {
-      uint8_t* dst = reinterpret_cast<uint8_t*>(p_cpx) + nb * kb_x * BTILE_BYTES;
-      HY3D_CUDA(ctx, cudaMemcpyAsync(dst, reinterpret_cast<const uint8_t*>(p_cp) + nb * kb_o * BTILE_BYTES, kb_o * BTILE_BYTES,
-                                     cudaMemcpyDeviceToDevice, ctx->stream));
-      HY3D_CUDA(ctx, cudaMemcpyAsync(dst + kb_o * BTILE_BYTES, reinterpret_cast<const uint8_t*>(p_qp) + nb * 3 * BTILE_BYTES, 3 * BTILE_BYTES,
-                                     cudaMemcpyDeviceToDevice, ctx->stream));
-    }
+    const int kb_o = (int)W / 64;
+    if (int rc = build(w.cproj_w, (int)W, (int)W, (int)W, 0, p_cpx, kb_o + 3)) return rc;
+    if (int rc = build(w.qp_w, (int)W, 192, w.E, 1, p_cpx + (size_t)kb_o * (BTILE_BYTES / 2), kb_o + 3)) return rc;
     float* b_cpx = c12 + 64 + 4 * W;
     k_add_vec<<<(unsigned)((W + 255) / 256), 256, 0, ctx->stream>>>(w.cproj_b, w.qp_b, (int)W, b_cpx);
     HY3D_LAUNCH_CHECK(ctx);
@@ -1279,66 +1215,45 @@ static int decode_tc_impl(hy3d_ctx* ctx, const QuerySource& src_in, long long n,
     return hy3d_fail(ctx, HY3D_ERR_UNSUPPORTED, "tcgen05 path needs head_dim 64 and widths that are multiples of 256");
   const int W = w.W, H = w.H, R = w.R;
   const int S = ST_PER_TILE * (W / BN);                         // statistic slots per row (one per 64 output columns)
-  const long long CH = ctx->chunk_points;                      // points per chunk (multiple of 256: whole CTA-pair tiles)
+  // points per chunk (a multiple of 256: whole CTA-pair tiles); the activations of one chunk are what the stages hand over
+  // through L2 / HBM.  131072 measured 1 % slower, 32768 7 % slower.
+  const long long CH = 262144;
   const long long chmax = n < CH ? (n + 127) / 128 * 128 : CH;
   HY3D_CUDA(ctx, ctx->ws[2].reserve((size_t)chmax * W * 4));          // R32 residual stream
-  HY3D_CUDA(ctx, ctx->ws[3].reserve((size_t)chmax * W * 2));          // T16 a (embed / raw x0 / attn out)
-  HY3D_CUDA(ctx, ctx->ws[4].reserve((size_t)chmax * W * 2));          // T16 q, then raw x1
+  HY3D_CUDA(ctx, ctx->ws[3].reserve((size_t)chmax * W * 2));          // T16 q, then raw x1
+  HY3D_CUDA(ctx, ctx->ws[4].reserve((size_t)chmax * W * 2));          // T16 attention output
   HY3D_CUDA(ctx, ctx->ws[5].reserve((size_t)chmax * W * R * 2));      // T16 h
-  HY3D_CUDA(ctx, ctx->ws[9].reserve((size_t)chmax * S * 7 * 4));      // row statistics: x0 (2), x1 (2), x2 (3) per slot
+  HY3D_CUDA(ctx, ctx->ws[9].reserve((size_t)chmax * S * 5 * 4));      // row statistics: x1 (2), x2 (3) per slot
   HY3D_CUDA(ctx, ctx->ws[6].reserve((size_t)chmax * 192 * 2));        // T16 Fourier features [hi | lo | hi] (kept for the fused c_proj)
-  // x0 stays out of HBM unless the per-stage activations are being retained for diagnostics
-  const bool fuse_x0 = !ctx->debug_retain && !(ctx->xbits & 0x80);
+  HY3D_CUDA(ctx, ctx->ln_mr.reserve((size_t)chmax * sizeof(float2)));  // ln_1 statistics of x0 (k_embed_tc)
   float* x = ctx->ws[2].as<float>();
   uint8_t* ta = ctx->ws[3].as<uint8_t>();
   uint8_t* tq = ctx->ws[4].as<uint8_t>();
   uint8_t* th = ctx->ws[5].as<uint8_t>();
   uint8_t* te = ctx->ws[6].as<uint8_t>();
-  float* st1 = ctx->ws[9].as<float>();
-  float* st3 = st1 + (size_t)chmax * S * 2;
+  float* st3 = ctx->ws[9].as<float>();
   float* stp = st3 + (size_t)chmax * S * 2;
   const float pi_mul = w.include_pi ? 3.14159265358979323846f : 1.f;
   for (long long p0 = 0; p0 < n; p0 += CH) {
     const long long P = (n - p0 < CH) ? (n - p0) : CH;
     const int Pb = (int)((P + 127) / 128);
-    const long long Pp = (long long)Pb * 128;
     QuerySource src = src_in;
     if (src.mode == 0) src.xyz += 3 * p0;
     else if (src.mode == 1) src.first += p0;
     else src.index += p0;
+    // q = q_norm(c_q(ln_1(query_proj(e)))) * scale * log2e as ONE K = 192 GEMM: c_q . query_proj collapsed into Wc (the
+    // LayerNorm between them only scales and shifts rows; its statistics are closed forms in e, computed by the embed
+    // kernel).  x0 is never formed, q is fp32-grade (x0 used to be rounded to fp16 on its way into c_q).
+    QStats qs{w.qs_wbar, w.qs_hc, w.qs_Gc, w.qs_scal, w.E};
+    HY3D_PROF(ctx, FAM_EMBED);
+    if (w.F == 8) k_embed_tc<8><<<(Pb < ctx->num_sms * 8 ? Pb : ctx->num_sms * 8), 128, 0, ctx->stream>>>(src, P, w.F, pi_mul, te, qs, 1e-6f, ctx->ln_mr.as<float2>());
+    else k_embed_tc<0><<<(Pb < ctx->num_sms * 8 ? Pb : ctx->num_sms * 8), 128, 0, ctx->stream>>>(src, P, w.F, pi_mul, te, qs, 1e-6f, ctx->ln_mr.as<float2>());
+    HY3D_LAUNCH_CHECK(ctx);
     GemmTC g{};
-    if (fuse_x0) {
-      // q = q_norm(c_q(ln_1(query_proj(e)))) * scale * log2e as ONE K = 192 GEMM: c_q . query_proj collapsed into Wc (the
-      // LayerNorm between them only scales and shifts rows; its statistics are closed forms in e, computed by the embed
-      // kernel).  x0 is never formed, q is fp32-grade (x0 used to be rounded to fp16 on its way into c_q).
-      HY3D_CUDA(ctx, ctx->ln_mr.reserve((size_t)chmax * sizeof(float2)));
-      QStats qs{w.qs_wbar, w.qs_hc, w.qs_Gc, w.qs_scal, w.E};
-      HY3D_PROF(ctx, FAM_EMBED);
-      if (w.F == 8) k_embed_tc<8><<<(Pb < ctx->num_sms * 8 ? Pb : ctx->num_sms * 8), 128, 0, ctx->stream>>>(src, P, w.F, pi_mul, te, qs, 1e-6f, ctx->ln_mr.as<float2>());
-      else k_embed_tc<0><<<(Pb < ctx->num_sms * 8 ? Pb : ctx->num_sms * 8), 128, 0, ctx->stream>>>(src, P, w.F, pi_mul, te, qs, 1e-6f, ctx->ln_mr.as<float2>());
-      HY3D_LAUNCH_CHECK(ctx);
-      g.Mb = Pb; g.A = te; g.B = reinterpret_cast<const uint8_t*>(w.t_cqx); g.KB = 3; g.N = W; g.Nb = W / BN; g.bias = w.bb_q; g.Tout = ta;
-      g.ln_mr = ctx->ln_mr.as<float2>(); g.cs = w.cs_qx; g.ln_eps = 1e-6f;
-      g.qn_w = w.qn_w; g.qn_b = w.qn_b; g.qk_norm = w.qk_norm ? 1 : 0; g.qscale = rsqrtf((float)w.D) * LOG2E;
-      if (int rc = launch_gemm<EPI_Q>(ctx, g, FAM_GEMM_CQ)) return rc;
-    } else {
-      HY3D_PROF(ctx, FAM_EMBED);
-      k_embed_tc<0><<<(Pb < ctx->num_sms * 8 ? Pb : ctx->num_sms * 8), 128, 0, ctx->stream>>>(src, P, w.F, pi_mul, te, QStats{}, 0.f, nullptr);
-      HY3D_LAUNCH_CHECK(ctx);
-      // (diagnostics: activations retained per stage) x0 = query_proj(e): fp32 residual, raw fp16 copy, row statistics
-      g.Mb = Pb; g.A = te; g.B = reinterpret_cast<const uint8_t*>(w.t_qp); g.KB = 3; g.N = W; g.Nb = W / BN; g.bias = w.qp_b;
-      g.Rout = x; g.Tcopy = tq; g.st_out = st1; g.st_k = 2;
-      if (int rc = launch_gemm<EPI_X0>(ctx, g, FAM_GEMM_QPROJ)) return rc;
-      if (int rc = hy3d_debug_keep(ctx, 0, x, (size_t)Pp * W * 4, 1, Pp, W)) return rc;
-      if (int rc = hy3d_debug_keep(ctx, 1, tq, (size_t)Pp * W * 2, 2, Pp, W)) return rc;
-      // q = q_norm(c_q(ln_1 x0)) * scale * log2e      (ln_1 folded: raw x0 operand, statistics applied in the epilogue)
-      g = GemmTC{}; g.Mb = Pb;
-      g.A = tq; g.B = reinterpret_cast<const uint8_t*>(w.t_cq); g.KB = W / 64; g.N = W; g.Nb = W / BN; g.bias = w.bb_q; g.Tout = ta;
-      g.st_in = st1; g.st_slots = S; g.st_np = ST_COLS; g.cs = w.cs_q; g.ln_eps = 1e-6f;
-      g.qn_w = w.qn_w; g.qn_b = w.qn_b; g.qk_norm = w.qk_norm ? 1 : 0; g.qscale = rsqrtf((float)w.D) * LOG2E;
-      if (int rc = launch_gemm<EPI_Q>(ctx, g, FAM_GEMM_CQ)) return rc;
-    }
-    if (int rc = hy3d_debug_keep(ctx, 2, ta, (size_t)Pp * W * 2, 2, Pp, W)) return rc;
+    g.Mb = Pb; g.A = te; g.B = reinterpret_cast<const uint8_t*>(w.t_cqx); g.KB = 3; g.N = W; g.Nb = W / BN; g.bias = w.bb_q; g.Tout = ta;
+    g.ln_mr = ctx->ln_mr.as<float2>(); g.cs = w.cs_qx; g.ln_eps = 1e-6f;
+    g.qn_w = w.qn_w; g.qn_b = w.qn_b; g.qk_norm = w.qk_norm ? 1 : 0; g.qscale = rsqrtf((float)w.D) * LOG2E;
+    if (int rc = launch_gemm<EPI_Q>(ctx, g, FAM_GEMM_CQ)) return rc;
     {
       AttnTC a{};
       a.Q = ta; a.O = tq; a.Pb = Pb; a.H = H;
@@ -1350,31 +1265,23 @@ static int decode_tc_impl(hy3d_ctx* ctx, const QuerySource& src_in, long long n,
       }
       if (int rc = launch_attn(ctx, a, w.attn_fast, FAM_ATTN, ctx->kv.shifted)) return rc;
     }
-    if (int rc = hy3d_debug_keep(ctx, 3, tq, (size_t)Pp * W * 2, 2, Pp, W)) return rc;
-    // x1 = x0 + c_proj(attn): fp32 residual in place + raw fp16 copy + statistics for the folded ln_3
+    // x1 = x0 + c_proj(attn) = [attn | e] [W_o | W_qp]^T + (b_o + b_qp): K-concatenated, no fp32 x0 in memory;
+    // fp32 residual + raw fp16 copy + statistics for the folded ln_3
     g = GemmTC{}; g.Mb = Pb;
-    if (fuse_x0) {       // [attn | e] [W_o | W_qp]^T + (b_o + b_qp): K-concatenated, no fp32 x0 in memory
-      g.A = tq; g.KB1 = W / 64; g.A2 = te; g.KB = W / 64 + 3; g.B = reinterpret_cast<const uint8_t*>(w.t_cpx); g.bias = w.b_cpx;
-    } else {
-      g.A = tq; g.KB = W / 64; g.B = reinterpret_cast<const uint8_t*>(w.t_cproj); g.bias = w.cproj_b; g.Rin = x;
-    }
+    g.A = tq; g.KB1 = W / 64; g.A2 = te; g.KB = W / 64 + 3; g.B = reinterpret_cast<const uint8_t*>(w.t_cpx); g.bias = w.b_cpx;
     g.N = W; g.Nb = W / BN; g.Rout = x; g.Tcopy = ta; g.st_out = st3; g.st_k = 2;
     if (int rc = launch_gemm<EPI_RES>(ctx, g, FAM_GEMM_CPROJ)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 4, x, (size_t)Pp * W * 4, 1, Pp, W)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 5, ta, (size_t)Pp * W * 2, 2, Pp, W)) return rc;
     // h = gelu(c_fc(ln_3 x1))                      (ln_3 folded)
     g = GemmTC{}; g.Mb = Pb;
     g.A = ta; g.B = reinterpret_cast<const uint8_t*>(w.t_fc); g.KB = W / 64; g.N = W * R; g.Nb = W * R / BN; g.bias = w.bb_fc; g.Tout = th;
     g.st_in = st3; g.st_slots = S; g.st_np = ST_COLS; g.cs = w.cs_fc; g.ln_eps = 1e-6f;
     if (int rc = launch_gemm<EPI_GELU>(ctx, g, FAM_GEMM_FC)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 6, th, (size_t)Pp * W * R * 2, 2, Pp, W * R)) return rc;
-    // x2 = x1 + c_proj(h): never stored (unless debugging) — only its row statistics and its dot with
-    // gamma_post * w_out, from which k_head_final forms [ln_post] + output_proj
+    // x2 = x1 + c_proj(h): never stored — only its row statistics and its dot with gamma_post * w_out, from which
+    // k_head_final forms [ln_post] + output_proj
     g = GemmTC{}; g.Mb = Pb;
     g.A = th; g.B = reinterpret_cast<const uint8_t*>(w.t_mp); g.KB = W * R / 64; g.N = W; g.Nb = W / BN; g.bias = w.mp_b;
-    g.Rin = x; g.Rout = ctx->debug_retain ? x : nullptr; g.st_out = stp; g.st_k = 3; g.dotw = w.dotw;
+    g.Rin = x; g.st_out = stp; g.st_k = 3; g.dotw = w.dotw;
     if (int rc = launch_gemm<EPI_RES>(ctx, g, FAM_GEMM_MLP)) return rc;
-    if (int rc = hy3d_debug_keep(ctx, 7, x, (size_t)Pp * W * 4, 1, Pp, W)) return rc;
     float* outp = d_out + (out_mode == 0 ? p0 : 0);
     HY3D_PROF(ctx, FAM_HEAD);
     k_head_final<<<Pb, 128, 0, ctx->stream>>>(stp, S, ST_COLS, w.ln_post ? 1 : 0, w.c12, src, P, outp, out_mode);
@@ -1629,16 +1536,6 @@ extern "C" int hy3d_transformer_forward(hy3d_ctx* ctx, const float* d_z, int32_t
     if (int rc = hy3d_transformer_layer_rest(ctx, l, t.kt.p)) return rc;
   }
   return hy3d_transformer_end(ctx, d_out);
-}
-
-extern "C" int hy3d_debug_timers(hy3d_ctx* ctx, uint64_t h_out[32]) {
-  if (!ctx || !h_out) return HY3D_ERR_ARG;
-  HY3D_CUDA(ctx, cudaSetDevice(ctx->device));
-  HY3D_CUDA(ctx, cudaStreamSynchronize(ctx->stream));
-  HY3D_CUDA(ctx, cudaMemcpyFromSymbol(h_out, hy3d_tm, sizeof(unsigned long long) * 32));
-  unsigned long long zero[32] = {};
-  HY3D_CUDA(ctx, cudaMemcpyToSymbol(hy3d_tm, zero, sizeof(zero)));
-  return HY3D_OK;
 }
 
 int hy3d_watchdog_enqueue(hy3d_ctx* ctx) {

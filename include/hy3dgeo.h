@@ -337,7 +337,7 @@ int hy3d_mc_cases(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n1, in
 /* ---- measurement ----------------------------------------------------------------------- */
 /* Device timing per kernel family with CUDA events recorded on the launch stream around every
  * launch (enable=1).  hy3d_profile_read synchronises, returns and clears the totals:
- * h_ms[f] milliseconds and h_count[f] launches of family f.  Families: 0 embed, 1 gemm query_proj,
+ * h_ms[f] milliseconds and h_count[f] launches of family f.  Families: 0 embed, 1 gemm query_proj (no longer emitted),
  * 2 layernorm, 3 gemm c_q, 4 attention, 5 gemm c_proj, 6 gemm c_fc, 7 gemm mlp.c_proj, 8 head,
  * 9 mc bits, 10 mc rowcount, 11 mc scan, 12 mc emit, 13 octree, 14 kv prepare, 15 kv select. */
 int hy3d_profile(hy3d_ctx* ctx, int enable);
@@ -348,28 +348,13 @@ int hy3d_profile_read(hy3d_ctx* ctx, double h_ms[16], int64_t h_count[16]);
  * h_out[0] != 0 means an mbarrier wait timed out inside a tcgen05 kernel (results of that
  * launch are invalid); h_out[1..4] = block, thread, barrier shared address, parity. */
 int hy3d_debug_watchdog(hy3d_ctx* ctx, int32_t h_out[8]);
-/* Keep (enable=1) the per-stage activations of the last decoded chunk for hy3d_debug_fetch.
- * Stage ids: 0 x0, 1 ln_1(x0), 2 q after q_norm (the tcgen05 path stores q*scale*log2e),
- * 3 attention output, 4 x1, 5 ln_3(x1), 6 MLP hidden, 7 x2.  Costs one device copy per stage. */
-int hy3d_debug_retain(hy3d_ctx* ctx, int enable);
-/* Kernel-tuning experiments (tools/gpu_chain_bench.py): `bits` disables parts of the tcgen05 kernels
- * (1 GEMM epilogue, 2 GEMM MMAs, 4 GEMM epilogue stores) so that their cost can be measured by difference — results
- * are garbage while those are set; 0x20 forces the online-softmax attention kernel, 0x40 runs the instrumented
- * bounded-score attention kernel (hy3d_debug_timers), 0x10000 the CUDA-core K/V projection (results stay valid);
- * 0x100 gives every attention stream its own K/V ring even when all query tiles share one K/V set;
- * `attn_poly` = pairs of every 8 pairs of attention exponentials evaluated as packed polynomials on the FMA pipe
- * (0 none, 1 .. 6 = that many pairs, 8 = all; other values select the default, 2 = a quarter of the exponentials).
- * Defaults (0, 2) are the product configuration. */
-int hy3d_debug_experiment(hy3d_ctx* ctx, int bits, int attn_poly);
-/* Phase clocks accumulated by the instrumented attention kernel (experiment bit 0x40), returned and cleared:
- * per head stream a (0, 1) h_out[8a + i] = SM cycles one softmax thread of CTA 0 spent in phase i
- * (0 wait S, 1 load S, 2 exponentials, 3 wait PV, 4 store P, 5 finalize), h_out[8a + 7] = KV tiles. */
-int hy3d_debug_timers(hy3d_ctx* ctx, uint64_t h_out[32]);
+/* enable=1: every tcgen05 attention launch of this context (decoder and latent transformer) runs the online-softmax
+ * kernel, also where the scores are bounded and the bounded-score kernel would run; hy3d_attention_info reports it.
+ * For tests that check both kernels against a reference.  enable=0 (the default) restores the automatic choice. */
+int hy3d_debug_force_online_softmax(hy3d_ctx* ctx, int enable);
 /* (query tile, head pair) items the exact redo pass recomputed after the LAST bounded-score attention launch with per-head
  * shifts (normally 0; see hy3d_attention_info).  Synchronises the stream. */
 int hy3d_debug_attn_redo(hy3d_ctx* ctx, int32_t* h_items);
-/* Row-major fp32 [rows, *h_width] copy of a retained stage, whatever its internal layout. */
-int hy3d_debug_fetch(hy3d_ctx* ctx, int stage, float* d_out, int64_t rows, int32_t* h_width);
 
 #ifdef __cplusplus
 }

@@ -127,13 +127,13 @@ def test_slab_partition_covers_every_plane_once():
     assert MC_HALO == 2                                              # hy3d_mc_count_slab: ids of the first halo plane need the second
 
 
-def test_new_entry_points_are_bound():
-    """Every slab / tuning entry point of include/hy3dgeo.h has a ctypes signature in the host wrapper."""
+def test_slab_and_debug_entry_points_are_bound():
+    """Every slab / debug entry point of include/hy3dgeo.h has a ctypes signature in the host wrapper and is exported."""
     from hy3dgeo import _lib
-    for name in ("hy3d_mc_count_slab", "hy3d_mc_emit_slab", "hy3d_transformer_forward", "hy3d_debug_experiment", "hy3d_debug_timers"):
+    for name in ("hy3d_mc_count_slab", "hy3d_mc_emit_slab", "hy3d_transformer_forward", "hy3d_debug_force_online_softmax"):
         assert name in _lib._SIGNATURES if hasattr(_lib, "_SIGNATURES") else True
     lib = _lib.load_library()
-    for name in ("hy3d_mc_count_slab", "hy3d_mc_emit_slab", "hy3d_debug_experiment", "hy3d_debug_timers"):
+    for name in ("hy3d_mc_count_slab", "hy3d_mc_emit_slab", "hy3d_debug_force_online_softmax"):
         assert getattr(lib, name) is not None
 
 

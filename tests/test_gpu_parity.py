@@ -311,7 +311,7 @@ def test_smoke_entry():
 
 # ---------------------------------------------------------------------------------- latent transformer
 @pytest.mark.parametrize("tag", ["mini", "full"])
-def test_latent_transformer_matches_oracle(tag, dev, ctx):
+def test_latent_transformer_matches_oracle_on_both_attention_kernels(tag, dev, ctx):
     """ShapeVAE.forward (reference model.py:186-189; post_kl + 16 pre-LN blocks) on the tcgen05 kernels
     (3-term split GEMMs, folded LayerNorms, fp16 self-attention) vs the fp32 CPU oracle: |latent| <= 6,
     max error < 1e-3 (measured 3.4e-4), rms < 2e-4 (measured 7e-5); both attention kernels."""
@@ -322,14 +322,14 @@ def test_latent_transformer_matches_oracle(tag, dev, ctx):
     ref = OD.shapevae_forward(sd, z, cfg.heads)
     vae = hy3dgeo.B200ShapeVAE(cfg, sd, device=dev)
     try:
-        for bits in (0, 0x20):                       # bounded-score kernel (default for these norms), online-softmax kernel
-            ctx.debug_experiment(bits, 2)
+        for online in (False, True):                 # bounded-score kernel (default for these norms), online-softmax kernel
+            ctx.debug_force_online_softmax(online)
             lat = vae(z.to(dev)).cpu()
             ctx.check_watchdog()
             d = (lat - ref).abs()
             assert lat.shape == ref.shape and float(d.max()) < 1e-3 and float(d.pow(2).mean().sqrt()) < 2e-4
     finally:
-        ctx.debug_experiment(0, 2)
+        ctx.debug_force_online_softmax(False)
 
 
 # ---------------------------------------------------------------------------------- FlashVDM

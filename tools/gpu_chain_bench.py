@@ -1,9 +1,8 @@
 #!/usr/bin/env python3
 """Per-kernel-family device time of the tcgen05 decoder chain on a fixed list of query points
-(full model unless --model mini).  With HY3D_DBG set (experiment bits, decoder_tc.cu) the results are
-garbage and only the timings mean anything.
+(full model unless --model mini).
 
-    [HY3D_DBG=bits] python tools/gpu_chain_bench.py [--points 524288] [--reps 3] [--tag name]
+    python tools/gpu_chain_bench.py [--points 524288] [--reps 3] [--tag name]
 """
 import argparse, json, os, sys
 import numpy as np, torch
@@ -19,8 +18,6 @@ ap.add_argument("--points", type=int, default=524288)
 ap.add_argument("--reps", type=int, default=3)
 ap.add_argument("--tag", default="")
 ap.add_argument("--no-pre", action="store_true", help="skip the transformer / K/V timings (short kernel sequence for ncu)")
-ap.add_argument("--bits", default="0", help="comma list of experiment bit sets")
-ap.add_argument("--poly", default="2", help="comma list of attn_poly values (2 = product default: a quarter of the exponentials as polynomials)")
 args = ap.parse_args()
 dev = torch.device("cuda:0")
 cfg = W.FULL if args.model == "full" else W.MINI
@@ -42,50 +39,28 @@ def timed(fn, reps=5):
     return a.elapsed_time(b) / reps
 if not args.no_pre:
     pre = {"transformer_ms": round(timed(lambda: vae(z)), 3)}
-    ctx.debug_experiment(0x10000, 0); pre["prepare_kv_simt_ms"] = round(timed(lambda: ctx.prepare_kv(lat[0])), 3)
-    ctx.debug_experiment(0, 0); pre["prepare_kv_tc_ms"] = round(timed(lambda: ctx.prepare_kv(lat[0])), 3)
+    pre["prepare_kv_ms"] = round(timed(lambda: ctx.prepare_kv(lat[0])), 3)
     print(json.dumps(pre), flush=True)
 M, Wd, R = cfg.num_latents, cfg.width, 4
-flops = {"gemm_query_proj": 2 * 51 * Wd, "gemm_c_q": 2 * Wd * Wd, "attention": 4 * M * Wd, "gemm_c_proj": 2 * Wd * Wd,
+flops = {"gemm_c_q": 2 * Wd * Wd, "attention": 4 * M * Wd, "gemm_c_proj": 2 * Wd * Wd,
          "gemm_c_fc": 2 * R * Wd * Wd, "gemm_mlp_proj": 2 * R * Wd * Wd}
-for bits in [int(b) for b in args.bits.split(",")]:
-    for poly in [int(b) for b in args.poly.split(",")]:
-        ctx.debug_experiment(bits, poly)
-        for _ in range(2):
-            out = ctx.decode_points(xyz)
-        torch.cuda.synchronize()
-        ctx.profile_read(); ctx.profile(True); ctx.debug_timers()
-        e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
-        e0.record()
-        for _ in range(args.reps):
-            out = ctx.decode_points(xyz)
-        e1.record(); torch.cuda.synchronize()
-        prof = ctx.profile_read(); ctx.profile(False)
-        wd = ctx.watchdog()
-        res = {"tag": args.tag, "bits": bits, "poly": poly, "points": args.points, "total_ms": round(e0.elapsed_time(e1) / args.reps, 3),
-               "watchdog": int(wd[0]), "families": {}}
-        for f, (ms, cnt) in prof.items():
-            if cnt:
-                d = {"ms": round(ms / args.reps, 3)}
-                if f in flops:
-                    d["tflops"] = round(flops[f] * args.points / (ms / args.reps) / 1e9, 1)
-                res["families"][f] = d
-        if bits & 8:        # SM clock during each GEMM family = cycles of CTA 0 / device time
-            tm = ctx.debug_timers()
-            n = max(tm[19], 1)  # all GEMM launches pooled: cycles per pair-tile of the leader MMA warp / one epilogue warp
-            res["gemm_clk_per_tile"] = {"mma_wait_tempty": round(tm[16] / n), "mma_wait_full": round(tm[17] / n), "mma_issue": round(tm[18] / n),
-                                        "epi_wait_tfull": round(tm[20] / n), "epi_work": round(tm[21] / n)}
-            fam_of = {0: "gemm_query_proj", 1: "gemm_c_q", 3: "gemm_c_fc"}
-            for epi, fam in fam_of.items():
-                if fam in res["families"] and tm[24 + epi]:
-                    res["families"][fam]["sm_mhz"] = round(tm[24 + epi] / args.reps / (res["families"][fam]["ms"] * 1e3))
-            if tm[26]:      # EPI_RES: c_proj + mlp_proj together
-                ms = res["families"]["gemm_c_proj"]["ms"] + res["families"]["gemm_mlp_proj"]["ms"]
-                res["families"]["gemm_mlp_proj"]["sm_mhz_res"] = round(tm[26] / args.reps / (ms * 1e3))
-        if bits & 0x40:
-            tm = ctx.debug_timers()
-            res["softmax_clk_per_tile"] = [[round(tm[8 * a + i] / max(tm[8 * a + 7], 1)) for i in range(6)] for a in range(2)]
-            # MMA warp of each stream: cycles per KV tile waiting for the K tile, the S buffer, the V tile, the stored P
-            res["mma_wait_clk_per_tile"] = [[round(tm[16 + 4 * a + i] / max(tm[8 * a + 7], 1)) for i in range(4)] for a in range(2)]
-        print(json.dumps(res), flush=True)
-ctx.debug_experiment(0, 2)
+for _ in range(2):
+    out = ctx.decode_points(xyz)
+torch.cuda.synchronize()
+ctx.profile_read(); ctx.profile(True)
+e0, e1 = torch.cuda.Event(enable_timing=True), torch.cuda.Event(enable_timing=True)
+e0.record()
+for _ in range(args.reps):
+    out = ctx.decode_points(xyz)
+e1.record(); torch.cuda.synchronize()
+prof = ctx.profile_read(); ctx.profile(False)
+wd = ctx.watchdog()
+res = {"tag": args.tag, "points": args.points, "total_ms": round(e0.elapsed_time(e1) / args.reps, 3), "watchdog": int(wd[0]),
+       "families": {}}
+for f, (ms, cnt) in prof.items():
+    if cnt:
+        d = {"ms": round(ms / args.reps, 3)}
+        if f in flops:
+            d["tflops"] = round(flops[f] * args.points / (ms / args.reps) / 1e9, 1)
+        res["families"][f] = d
+print(json.dumps(res), flush=True)
