@@ -63,6 +63,7 @@ SYMBOLS = {
     "hy3d_set_stream": (C.c_int, [C.c_void_p, C.c_void_p]),
     "hy3d_last_error": (C.c_char_p, [C.c_void_p]),
     "hy3d_set_precision": (C.c_int, [C.c_void_p, C.c_int]),
+    "hy3d_set_mc_face_rule": (C.c_int, [C.c_void_p, C.c_int]),
     "hy3d_launch_count": (C.c_int64, [C.c_void_p]),
     "hy3d_attention_info": (C.c_int, [C.c_void_p, C.POINTER(C.c_float), C.POINTER(C.c_int32), C.POINTER(C.c_float)]),
     "hy3d_set_decoder_weights": (C.c_int, [C.c_void_p, C.POINTER(DecoderDesc)]),
@@ -148,6 +149,11 @@ def load_library():
                 fn.argtypes = args
             _lib = lib
     return _lib
+
+
+# marching cubes, ambiguous faces (hy3dgeo.h hy3d_set_mc_face_rule): "sign" separates the inside corners, "asymptotic"
+# decides from the four values as scikit-image's Lewiner face test does
+MC_FACE_RULES = {"sign": 0, "asymptotic": 1}
 
 
 class Hy3dError(RuntimeError):
@@ -548,8 +554,15 @@ class GeoContext:
                     "hy3d_sentinel_to_nan")
 
     # ---- marching cubes ------------------------------------------------------------------------
-    def mc_count(self, grid: torch.Tensor, level: float):
+    def set_mc_face_rule(self, rule: str):
+        """Ambiguous-face rule of the next count / emit pair, a name of MC_FACE_RULES (mc_count and mc_count_slab set it)."""
+        if rule not in MC_FACE_RULES:
+            raise ValueError(f"face_rule must be one of {sorted(MC_FACE_RULES)}, got {rule!r}")
+        self._check(self.lib.hy3d_set_mc_face_rule(self.h, MC_FACE_RULES[rule]), "hy3d_set_mc_face_rule")
+
+    def mc_count(self, grid: torch.Tensor, level: float, face_rule: str = "sign"):
         self.sync_stream()
+        self.set_mc_face_rule(face_rule)
         nv, nf = C.c_int64(), C.c_int64()
         mm = (C.c_float * 3)()
         self._check(self.lib.hy3d_mc_count(self.h, _ptr(grid), grid.shape[0], grid.shape[1], grid.shape[2], float(level),
@@ -563,9 +576,10 @@ class GeoContext:
         a = (C.c_double * 3)(*[float(v) for v in add])
         self._check(self.lib.hy3d_mc_emit(self.h, d, m, a, _ptr(verts), _ptr(faces)), "hy3d_mc_emit")
 
-    def mc_count_slab(self, grid: torch.Tensor, own_planes: int, level: float):
+    def mc_count_slab(self, grid: torch.Tensor, own_planes: int, level: float, face_rule: str = "sign"):
         """grid = owned planes followed by the next slab's halo planes; counts of the owned part (see hy3dgeo.h)."""
         self.sync_stream()
+        self.set_mc_face_rule(face_rule)
         nv, nf = C.c_int64(), C.c_int64()
         mm = (C.c_float * 3)()
         self._check(self.lib.hy3d_mc_count_slab(self.h, _ptr(grid), grid.shape[0], grid.shape[1], grid.shape[2], int(own_planes),

@@ -122,6 +122,13 @@ int hy3d_set_precision(hy3d_ctx* ctx, int precision) {
   return HY3D_OK;
 }
 
+int hy3d_set_mc_face_rule(hy3d_ctx* ctx, int rule) {
+  if (!ctx) return HY3D_ERR_ARG;
+  if (rule != HY3D_MC_FACE_SIGN && rule != HY3D_MC_FACE_ASYMPTOTIC) return hy3d_fail(ctx, HY3D_ERR_ARG, "unknown face rule %d", rule);
+  ctx->mc.rule = rule;
+  return HY3D_OK;
+}
+
 int64_t hy3d_launch_count(const hy3d_ctx* ctx) { return ctx ? ctx->launches : 0; }
 
 int hy3d_attention_info(hy3d_ctx* ctx, float* h_score_bound, int32_t* h_bounded_kernel, float* h_measured_bound) {

@@ -101,6 +101,8 @@ struct McState {
   int n0 = 0, n1 = 0, n2 = 0, words = 0;
   int own_planes = 0;                 // slab mode: planes [0, own_planes) are owned, the rest is the next slab's halo
   float level = 0.f;
+  int rule = HY3D_MC_FACE_SIGN;       // hy3d_set_mc_face_rule: applies to the next count / emit pair
+  int counted_rule = HY3D_MC_FACE_SIGN;   // the rule the last count ran under: an emit under another rule is refused
   long long nV = 0, nF = 0;
   DevBuf bits, rowcnt, rowoff, stats;
 };

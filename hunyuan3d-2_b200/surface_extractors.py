@@ -11,7 +11,7 @@ from typing import List, Tuple, Union
 import numpy as np
 import torch
 
-from ._lib import get_context
+from ._lib import MC_FACE_RULES, get_context
 
 
 def _to_host(*tensors):
@@ -71,17 +71,25 @@ class MCSurfaceExtractor(SurfaceExtractor):
     ``v / (res+1) * bbox_size + bbox_min`` evaluated in float64 on the device.  Only the
     mesh crosses PCIe (the reference copies the whole fp32 grid to the host, :70).
 
-    The marching cubes here is the classic 256-case table with one fixed sign rule for ambiguous faces, vertices in
-    lexicographic (voxel, axis) order — NOT scikit-image's Lewiner variant (no face / interior tests, different vertex and
-    face order): same surface up to the ambiguous-cube topology and the indexing, see INTEGRATION.md "marching cubes".
+    The marching cubes here is the classic 256-case table, vertices in lexicographic (voxel, axis) order — NOT
+    scikit-image's Lewiner variant (no interior tests, different vertex and face order): same surface up to the
+    ambiguous-cube topology and the indexing, see INTEGRATION.md "marching cubes".
+
+    ``face_rule`` decides ambiguous cube faces (two inside corners on one diagonal): ``"sign"`` (default) always separates
+    the inside corners; ``"asymptotic"`` connects them iff the product of their values (minus ``mc_level``) exceeds that of
+    the outside corners — Lewiner's face test, so thin parts resolve as skimage resolves them.  Same vertices either way;
+    both meshes are watertight.
 
     ``cull_nonfinite`` (default off = the reference's output, NaN vertices included): drop, on the device, the NaN / inf
     vertices the sparse decoders produce along the rim of their visited band, the faces that use them and any vertex left
     unreferenced — what ``trimesh.Trimesh(...)`` does on the host in the reference's next step (``export_to_trimesh``,
     pipelines.py:95-110), which then finds nothing to remove.  ``hy3dgeo.export_to_trimesh`` does cull + winding flip."""
 
-    def __init__(self, cull_nonfinite: bool = False):
+    def __init__(self, cull_nonfinite: bool = False, face_rule: str = "sign"):
+        if face_rule not in MC_FACE_RULES:
+            raise ValueError(f"face_rule must be one of {sorted(MC_FACE_RULES)}, got {face_rule!r}")
         self.cull_nonfinite = cull_nonfinite
+        self.face_rule = face_rule
 
     def run_device(self, grid_logit: torch.Tensor, *, mc_level, bounds, octree_resolution, **kwargs):
         """Returns device tensors (verts float32 [V,3], faces int32 [F,3])."""
@@ -99,7 +107,7 @@ class MCSurfaceExtractor(SurfaceExtractor):
             raise ValueError("Input volume should be a 3D numpy array.")
         grid = grid_logit.detach().to(torch.float32).contiguous()
         ctx = get_context(grid.device)
-        nv, nf, (vmin, vmax, has_nan) = ctx.mc_count(grid, mc_level)
+        nv, nf, (vmin, vmax, has_nan) = ctx.mc_count(grid, mc_level, self.face_rule)
         # skimage: level outside [min, max] -> ValueError; NaN in the volume disables the check
         if not has_nan and (mc_level < vmin or mc_level > vmax):
             raise ValueError("Surface level must be within volume data range.")
@@ -135,7 +143,7 @@ class MCSurfaceExtractor(SurfaceExtractor):
         if not isinstance(slab, torch.Tensor) or not slab.is_cuda:
             raise RuntimeError("MCSurfaceExtractor needs a CUDA tensor (hy3dgeo has no CPU path)")
         self._slab = slab.detach().to(torch.float32).contiguous()
-        return get_context(slab.device).mc_count_slab(self._slab, own_planes, mc_level)
+        return get_context(slab.device).mc_count_slab(self._slab, own_planes, mc_level, self.face_rule)
 
     def emit_slab(self, nv: int, nf: int, plane0: int, id_base: int, *, bounds, octree_resolution):
         """Vertices / faces of the slab counted last; face ids are global (id_base = vertices of all earlier slabs)."""

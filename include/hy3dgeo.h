@@ -252,6 +252,16 @@ int hy3d_mc_count_slab(hy3d_ctx* ctx, const float* d_grid, int32_t n0, int32_t n
                        int64_t* h_num_verts, int64_t* h_num_faces, float h_minmax[3]);
 int hy3d_mc_emit_slab(hy3d_ctx* ctx, const double h_div[3], const double h_mul[3], const double h_add[3], int32_t plane0,
                       int64_t id_base, float* d_verts, int32_t* d_faces);
+/* How marching cubes resolves an ambiguous cube face (two inside corners on one diagonal, two outside on the other).
+ * HY3D_MC_FACE_SIGN (default): the inside corners are always separated.  HY3D_MC_FACE_ASYMPTOTIC: the asymptotic decider of
+ * scikit-image's Lewiner face test -- with d = v - level in float32, inside diagonal (a, c) and outside diagonal (b, d), the
+ * inside corners connect iff (double)d_a * (double)d_c > (double)d_b * (double)d_d (equality or NaN: separated).  Both
+ * rules give watertight meshes with the same vertices; only the faces of cubes with an ambiguous face differ.  The rule
+ * applies to the next hy3d_mc_count[_slab] / hy3d_mc_emit[_slab] pair: an emit under a rule other than its count's returns
+ * HY3D_ERR_STATE.  An unknown rule returns HY3D_ERR_ARG. */
+#define HY3D_MC_FACE_SIGN 0
+#define HY3D_MC_FACE_ASYMPTOTIC 1
+int hy3d_set_mc_face_rule(hy3d_ctx* ctx, int rule);
 /* ---- dual marching cubes: replaces DMCSurfaceExtractor.run (surface_extractors.py:79-94), i.e. diso.DiffDMC(sdf =
  * -logits / res, normalize=True) + center_vertices (:29-34) + the reversed winding ------------------------------------
  * Phase 1: classify + count.  d_grid: fp32 [n0,n1,n2]; inside test `g > 0` (iso-value 0 of sdf = -logit / res), NaN =>

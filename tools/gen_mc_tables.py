@@ -8,7 +8,9 @@ resolved by one fixed rule that depends only on the four corner signs of that
 face — "inside corners are separated" — so the two cubes sharing a face always
 agree and the extracted surface is watertight (the classic Lorensen table is
 not).  skimage's Lewiner variant resolves those faces from the values instead;
-see DESIGN.md "marching cubes: parity unpinned".
+see DESIGN.md "marching cubes: parity unpinned".  For that value-based choice
+(the asymptotic decider, the opt-in `face_rule="asymptotic"`) the same tracing
+runs once per combination of per-face choices: mc_tables_decider.inc.
 
 Conventions (SURVEY Appendix D): cube corner m has offsets (dx,dy,dz) with
 x = array axis 2 (fastest), y = axis 1, z = axis 0:
@@ -16,10 +18,12 @@ x = array axis 2 (fastest), y = axis 1, z = axis 0:
 case bit m is set iff value(v_m) - level > 0.
 Edge e joins CORNER pairs EDGES[e]; the edge is *owned* by its lower corner.
 
-Output: hunyuan3d-2_b200/csrc/mc_tables.inc  (checked in; regenerate with
-`python tools/gen_mc_tables.py`).  The C oracle (oracle/mc_oracle.c) does NOT
-read this table: it traces loops at run time, so a parity test between the two
-checks the table.
+Output: hunyuan3d-2_b200/csrc/mc_tables.inc, dmc_tables.inc and
+mc_tables_decider.inc (checked in; regenerate with
+`python tools/gen_mc_tables.py [output directory]`).  The C oracles
+(oracle/mc_oracle.c, and oracle/mc_face_rule.c for the face rules) do NOT read
+these tables: they trace loops at run time, so a parity test between the two
+checks the tables.
 """
 import itertools
 import os
@@ -79,10 +83,11 @@ def face_segments(case, cyc, connect_inside=False):
     return segs
 
 
-def trace_loops(case, connect_inside=False):
+def trace_loops(case, connect=0):
+    """Iso-contour loops of one cube.  Bit f of `connect` set: ambiguous face FACES[f] connects its inside corners."""
     nxt = {}
-    for cyc in FACES:
-        for a, b in face_segments(case, cyc, connect_inside):
+    for f, cyc in enumerate(FACES):
+        for a, b in face_segments(case, cyc, bool((connect >> f) & 1)):
             assert a not in nxt
             nxt[a] = b
     loops, seen = [], set()
@@ -99,9 +104,9 @@ def trace_loops(case, connect_inside=False):
     return loops
 
 
-def triangles(case, flip):
+def triangles(case, flip, connect=0):
     tris = []
-    for loop in trace_loops(case):
+    for loop in trace_loops(case, connect):
         for m in range(1, len(loop) - 1):
             t = (loop[0], loop[m], loop[m + 1])
             tris.append((t[0], t[2], t[1]) if flip else t)
@@ -112,11 +117,72 @@ def build(flip=True):
     return [triangles(c, flip) for c in range(256)]
 
 
-def main():
+def ambiguous_faces(case):
+    """Indices into FACES of the faces whose inside corners are diagonal, ascending."""
+    out = []
+    for f, cyc in enumerate(FACES):
+        ins = [(case >> c) & 1 for c in cyc]
+        if ins[0] == ins[2] and ins[1] == ins[3] and ins[0] != ins[1]:
+            out.append(f)
+    return out
+
+
+def decision_connect(case, dec):
+    """Face mask for trace_loops from decision index `dec`: bit q of dec is the choice of the q-th ambiguous face."""
+    return sum(1 << f for q, f in enumerate(ambiguous_faces(case)) if (dec >> q) & 1)
+
+
+def build_decider(flip=True):
+    """Per case, 2^k triangle lists (k ambiguous faces), one per decision index."""
+    return [[triangles(c, flip, decision_connect(c, dec)) for dec in range(1 << len(ambiguous_faces(c)))] for c in range(256)]
+
+
+def write_decider_tables(out):
+    table = build_decider(flip=True)
+    assert all(rows[0] == tris for rows, tris in zip(table, build(flip=True)))     # no face connected: the sign-rule table
+    maxt = max(len(t) for rows in table for t in rows)
+    nrows = sum(len(rows) for rows in table)
+    with open(out, "w") as f:
+        f.write("// GENERATED by tools/gen_mc_tables.py — do not edit.\n")
+        f.write("// Marching cubes with the asymptotic decider on ambiguous faces.  Faces f = 0..5 (corner cycles\n")
+        f.write("// hy3d_mc_face_corner[f], counter-clockwise seen from outside).  Per case c: hy3d_mc_amb_faces[c] = mask of its\n")
+        f.write("// ambiguous faces (inside corners diagonal); with k of them, rows hy3d_mc_dec_first[c] + d, d = 0 .. 2^k - 1, of\n")
+        f.write("// hy3d_mc_dec_tri hold its triangles when bit q of d says whether the q-th ambiguous face (ascending f) connects its\n")
+        f.write("// inside corners.  Row d = 0 is the row of mc_tables.inc.  Row: triangle count, 3 edge ids per triangle, -1 padded.\n")
+        f.write(f"#define HY3D_MC_DEC_MAX_TRIS {maxt}\n")
+        f.write(f"#define HY3D_MC_DEC_ROW {1 + 3 * maxt}\n")
+        f.write(f"#define HY3D_MC_DEC_ROWS {nrows}\n")
+        f.write("HY3D_MC_DEC_QUAL signed char hy3d_mc_face_corner[6][4] = {\n")
+        f.write("  " + ",".join("{" + ",".join(str(c) for c in cyc) + "}" for cyc in FACES) + "};\n")
+        masks = [sum(1 << fc for fc in ambiguous_faces(c)) for c in range(256)]
+        f.write("HY3D_MC_DEC_QUAL unsigned char hy3d_mc_amb_faces[256] = {\n")
+        for c0 in range(0, 256, 32):
+            f.write("  " + ",".join(str(v) for v in masks[c0:c0 + 32]) + ",\n")
+        f.write("};\n")
+        first, acc = [], 0
+        for rows in table:
+            first.append(acc)
+            acc += len(rows)
+        f.write("HY3D_MC_DEC_QUAL short hy3d_mc_dec_first[256] = {\n")
+        for c0 in range(0, 256, 16):
+            f.write("  " + ",".join(str(v) for v in first[c0:c0 + 16]) + ",\n")
+        f.write("};\n")
+        f.write("HY3D_MC_DEC_QUAL signed char hy3d_mc_dec_tri[HY3D_MC_DEC_ROWS][HY3D_MC_DEC_ROW] = {\n")
+        for c, rows in enumerate(table):
+            for dec, tris in enumerate(rows):
+                row = [len(tris)] + [e for t in tris for e in t]
+                row += [-1] * (1 + 3 * maxt - len(row))
+                f.write("  {" + ",".join(f"{v:2d}" for v in row) + "},\n")
+        f.write("};\n")
+    print(f"wrote {os.path.normpath(out)}; {nrows} rows, max triangles per cube = {maxt}")
+
+
+def main(outdir=None):
     table = build(flip=True)
     maxt = max(len(t) for t in table)
     here = os.path.dirname(os.path.abspath(__file__))
-    out = os.path.join(here, "..", "hunyuan3d-2_b200", "csrc", "mc_tables.inc")
+    outdir = outdir or os.path.join(here, "..", "hunyuan3d-2_b200", "csrc")
+    out = os.path.join(outdir, "mc_tables.inc")
     with open(out, "w") as f:
         f.write("// GENERATED by tools/gen_mc_tables.py — do not edit.\n")
         f.write("// 256-case marching-cubes table derived by face-loop tracing (fixed ambiguous-face rule:\n")
@@ -141,7 +207,8 @@ def main():
         f.write("};\n")
     print(f"wrote {os.path.normpath(out)}; max triangles per cube = {maxt}")
     print("faces (ccw from outside):", FACES)
-    write_dmc_tables(os.path.join(here, "..", "hunyuan3d-2_b200", "csrc", "dmc_tables.inc"))
+    write_dmc_tables(os.path.join(outdir, "dmc_tables.inc"))
+    write_decider_tables(os.path.join(outdir, "mc_tables_decider.inc"))
 
 
 def dmc_patches(case):
@@ -177,4 +244,4 @@ def write_dmc_tables(out):
 
 
 if __name__ == "__main__":
-    main()
+    main(sys.argv[1] if len(sys.argv) > 1 else None)
